@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the BISIP MCMC likelihood hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): log-prob evals/sec = spectra x walkers x steps / time.
 Workload: BASELINE config 5 — Debye polynomial decomposition (poly_deg 4, 64 taus) of synthetic
@@ -24,8 +24,12 @@ mean / std summary, and for N>1 the NCCL all-gather of the summaries.
            alone, end to end, and a roofline fraction each.
 `strong_scaling`: the fixed 100,000-spectra survey through ONE `bisip_b200.fit_sharded` call on the N ranks.
 `cpu_baseline`: the reference's own Cython + NumPy log-probability (oracle/_ref) under the emcee
-           restatement, on all host cores, on a bounded sample of the same spectra.
+           restatement, on all host cores, on a bounded sample of the same spectra.  Where the reference package is not
+           built, the C restatement oracle/bisip_oracle.c runs instead; `note` says which of the two was timed.
 `--impl reference`: that CPU arm alone, as its own JSON line.
+`--dump-outputs DIR`: after the timed steps, what the last timed step computed goes to DIR/<name>.npy (float64): the
+           per-spectrum summaries and the kept chains of a fixed, seeded sample of spectra (see `dump_outputs`).  The
+           inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -85,6 +89,32 @@ def _ref_worker(args):
     return dt, m.get_param_mean(discard=nsteps // 2)
 
 
+def _restatement_worker(args):
+    """One process = one synthetic spectrum through the C restatement of the reference's log-probability and of
+    emcee's stretch move (oracle/bisip_oracle.c): the same posterior, walkers and steps as `_ref_worker`."""
+    b, zn, zn_err, w, walkers, nsteps = args
+    from bisip_b200.batch import default_bounds, tau_grid
+    from oracle import oracle
+    _, taus, log_taus = tau_grid(w, N_TAU, POLY_DEG)
+    _, bounds = default_bounds('decomp', POLY_DEG)
+    prob = oracle.Problem('decomp', w, zn, zn_err, bounds, taus=taus, log_taus=log_taus, c_exp=1.0)
+    p0 = np.random.default_rng(1000 + b).uniform(bounds[0], bounds[1], (walkers, bounds.shape[1]))
+    t0 = time.perf_counter()
+    prob.run(p0, nsteps, seed=SEED, spectrum=b)
+    return time.perf_counter() - t0
+
+
+def reference_impl():
+    """(worker, description) of the CPU arm.  The reference package is used where oracle/build_ref.sh built it into
+    oracle/_ref (that needs the reference's sources, which this repository does not hold); otherwise the repository's
+    own C restatement of it runs, so that the CPU arm works from a plain checkout."""
+    from oracle import refload
+    if refload.available():
+        return _ref_worker, "reference models.py + Cython (oracle/_ref) under oracle/emcee_restatement.py"
+    return _restatement_worker, ("C restatement of the reference's log-probability and emcee's stretch move "
+                                 "(oracle/bisip_oracle.c); the reference package (oracle/_ref) is not built")
+
+
 def reference_sample(zn, zn_err, w, cores, walkers=WALKERS, nsteps=None, pool=None):
     """Bounded sample: `cores` spectra (one per process) x walkers x nsteps.  Returns evals/s."""
     import multiprocessing as mp
@@ -94,7 +124,7 @@ def reference_sample(zn, zn_err, w, cores, walkers=WALKERS, nsteps=None, pool=No
     if own:
         pool = mp.get_context("fork").Pool(cores)
     t0 = time.perf_counter()
-    pool.map(_ref_worker, jobs)
+    pool.map(reference_impl()[0], jobs)
     wall = time.perf_counter() - t0
     if own:
         pool.close()
@@ -149,8 +179,7 @@ def run_reference(args):
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": {"workload": WORKLOAD, "sample_per_step": sample},
         "cpu_baseline": {"value": val, "unit": "evals/s", "cores": cores, "kind": kind, "sample": sample,
-                         "note": "reference models.py + Cython (oracle/_ref) driven by oracle/emcee_restatement.py; "
-                                 "the emcee package itself is not installable here"},
+                         "note": reference_impl()[1]},
         "e2e": {"value": val, "unit": "evals/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }))
 
@@ -357,6 +386,37 @@ def run_other_configs(torch, engine, synthetic, BatchInversion, _lib, dev, peak_
     return out
 
 
+DUMP_MAX_SPECTRA = 100_000     # per-spectrum summaries: 32 float64 each, 25.6 MB at most
+DUMP_CHAINS = 16               # kept chains of 16 spectra: 100 x 256 x 6 float64 each, 19.7 MB at the default shape
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(torch, path, out, res):
+    """Write what the last timed step computed, as float64 .npy files in `path`: the per-spectrum summaries of
+    `step_resident` (percentiles, mean, std, acceptance_fraction) and, for DUMP_CHAINS spectra, the kept chain and the
+    per-walker accepted counts of `engine.ensemble_run`.  Row sets are fixed by SEED (`spectra`, `chain_spectra` hold
+    the indices), so that runs with the same arguments write the same rows."""
+    rng = np.random.default_rng(SEED)
+    n = out['mean'].shape[0]
+    rows = np.arange(n) if n <= DUMP_MAX_SPECTRA else np.sort(rng.choice(n, DUMP_MAX_SPECTRA, replace=False))
+    crow = np.sort(rng.choice(res['chain'].shape[0], min(DUMP_CHAINS, res['chain'].shape[0]), replace=False))
+    arrays = {k: v[torch.from_numpy(rows).to(v.device)] for k, v in out.items()}
+    arrays["spectra"] = rows
+    sel = torch.from_numpy(crow).to(res['chain'].device)
+    arrays["chain"] = res['chain'][sel]
+    arrays["accepted"] = res['accepted'][sel]
+    arrays["chain_spectra"] = crow
+    arrays = {k: np.ascontiguousarray((v.cpu().numpy() if torch.is_tensor(v) else v), dtype=np.float64)
+              for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    print(f"bench: wrote {len(arrays)} arrays ({total / 2**20:.1f} MiB) to {path}", file=sys.stderr)
+
+
 def run_gpu(args):
     import torch
     import torch.distributed as dist
@@ -431,12 +491,15 @@ def run_gpu(args):
     barrier()
     t_ev0.record()
     for _ in range(args.steps):
+        res = None                  # the previous step's 15 GB chain is freed before the next one is allocated
         out, res = step_resident(True)
-        del res
     t_ev1.record()
     barrier()
     launches = _lib.launch_count() - launches0
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, out, res)
+    del res
     ms_total = t_ev0.elapsed_time(t_ev1)
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
@@ -454,7 +517,7 @@ def run_gpu(args):
     h2d = zn_h.numel() * 8 + ze_h.numel() * 8 + p0_h.numel() * 8 + syn['w'].nbytes
     e2e_ms = []
     d2h = 0
-    for i in range(max(1, min(args.steps, env_int("BISIP_BENCH_E2E_STEPS", 5)))):
+    for i in range(args.steps):
         barrier()
         t0 = time.perf_counter()
         r = inv.fit_gathered(B * world, p0=p0_h, discard=DISCARD, thin=THIN, percentiles=PCT)
@@ -587,7 +650,7 @@ def run_gpu(args):
             cpu_baseline = {"value": cpu_v, "unit": "evals/s", "cores": min(cores, B), "kind": "reference", "sample": cpu_sample,
                             "wall_s": cpu_wall, "evals_per_s_per_core": cpu_v / min(cores, B),
                             "extrapolated_days_for_full_config_on_these_cores": 1e5 * WALKERS * NSTEPS / cpu_v / 86400.0,
-                            "note": "reference models.py + Cython (oracle/_ref) under oracle/emcee_restatement.py"}
+                            "note": reference_impl()[1]}
             if env_int("BISIP_BENCH_CONFIGS", 1):
                 peak_dfma, _ = dfma_peak()
                 other = run_other_configs(torch, engine, synthetic, BatchInversion, _lib, dev, peak_sust, peak_dfma)
@@ -641,7 +704,11 @@ def main():
     ap.add_argument("--steps", type=int, default=3)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="graft", choices=["graft", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's results to DIR/<name>.npy (GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # convenience: `python bench.py --gpus N` re-launches itself one rank per GPU
         os.execvp(sys.executable, [sys.executable, "-m", "torch.distributed.run", "--nnodes=1",

@@ -386,6 +386,42 @@ def test_bench_reference_arm_prints_one_json_line():
     assert quiet.returncode == 0 and quiet.stdout == ''
 
 
+def test_bench_dump_outputs_writes_seeded_float64_samples(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: float64 .npy files whose sampled rows are fixed by the seed and equal the rows of the
+    step's results they name; the total is held under the limit."""
+    import importlib.util
+    import torch
+    spec = importlib.util.spec_from_file_location('bench_under_test', os.path.join(ROOT, 'bench.py'))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    monkeypatch.setattr(bench, 'DUMP_MAX_SPECTRA', 30)
+    g = torch.Generator().manual_seed(0)
+    B, W = 40, 8
+    out = {'percentiles': torch.rand(B, 3, 6, generator=g, dtype=torch.float64),
+           'mean': torch.rand(B, 6, generator=g, dtype=torch.float64),
+           'std': torch.rand(B, 6, generator=g, dtype=torch.float64),
+           'acceptance_fraction': torch.rand(B, generator=g, dtype=torch.float64)}
+    res = {'chain': torch.rand(B, 3, W, 6, generator=g, dtype=torch.float64),
+           'accepted': torch.randint(0, 100, (B, W), generator=g, dtype=torch.int32)}
+    bench.dump_outputs(torch, str(tmp_path / 'a'), out, res)
+    bench.dump_outputs(torch, str(tmp_path / 'b'), out, res)
+    names = sorted(os.listdir(tmp_path / 'a'))
+    assert names == sorted(f'{k}.npy' for k in list(out) + ['spectra', 'chain', 'accepted', 'chain_spectra'])
+    d = {n[:-4]: np.load(tmp_path / 'a' / n) for n in names}
+    for n in names:
+        assert d[n[:-4]].dtype == np.float64
+        np.testing.assert_array_equal(d[n[:-4]], np.load(tmp_path / 'b' / n))
+    rows, crow = d['spectra'].astype(int), d['chain_spectra'].astype(int)
+    assert len(rows) == 30 and np.all(np.diff(rows) > 0) and len(crow) == bench.DUMP_CHAINS and np.all(np.diff(crow) > 0)
+    for k in out:
+        np.testing.assert_array_equal(d[k], out[k].numpy()[rows])
+    np.testing.assert_array_equal(d['chain'], res['chain'].numpy()[crow])
+    np.testing.assert_array_equal(d['accepted'], res['accepted'].numpy()[crow])
+    monkeypatch.setattr(bench, 'DUMP_LIMIT', 1000)
+    with pytest.raises(ValueError):
+        bench.dump_outputs(torch, str(tmp_path / 'c'), out, res)
+
+
 _SHARDED_WORKER = r'''
 import os, sys
 sys.path.insert(0, os.environ["BISIP_ROOT"])
