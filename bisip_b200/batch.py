@@ -132,7 +132,7 @@ def gather_chain_to_rank0(chain, n_total, rank, world, group=None, chunk_bytes=1
 
 
 def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 97.5), p0=None, gather_chain=False,
-                group=None, batch_size=None, **kwargs):
+                group=None, batch_size=None, autocorr=False, **kwargs):
     """Invert a whole survey on all ranks of the current ``torch.distributed`` job (one process per GPU).
 
     The reference inverts a batch as a serial loop over files (``docs/tutorials/decomposition.ipynb`` cells 9-10);
@@ -140,9 +140,10 @@ def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 9
     (B, W, ndim)), inverts its contiguous block ``shard_range(B, rank, world)`` with ``BatchInversion`` (Philox
     counters carry the global spectrum index: the result does not depend on the number of ranks), and the
     per-spectrum summaries are all-gathered with one NCCL collective, so every rank returns the complete result:
-    ``percentiles`` (B, len(p), ndim), ``mean``, ``std`` (B, ndim), ``acceptance_fraction``, ``flags`` (B,).
-    With ``gather_chain=True`` the kept chains (``discard`` / ``thin``) are gathered to rank 0 in chunks
-    (``chain`` (B, n_keep, W, ndim) on rank 0, None elsewhere).  Without an initialised process group it runs the
+    ``percentiles`` (B, len(p), ndim), ``mean``, ``std`` (B, ndim), ``acceptance_fraction``, ``flags`` (B,), and with
+    ``autocorr=True`` ``autocorr_time`` (B, ndim) (see ``BatchInversion.fit``).  With ``gather_chain=True`` the kept
+    chains (``discard`` / ``thin``) are gathered to rank 0 in chunks (``chain`` (B, n_keep, W, ndim) on rank 0, None
+    elsewhere).  Without an initialised process group it runs the
     whole survey on the current device.  ``kwargs`` go to ``BatchInversion`` (nwalkers, nsteps, poly_deg, ...)."""
     import torch.distributed as dist
     on = dist.is_available() and dist.is_initialized()
@@ -153,7 +154,9 @@ def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 9
     w_arr = np.asarray(w, dtype=np.float64)
     inv = BatchInversion(model, w_arr if w_arr.ndim == 1 else w_arr[lo:hi], zn[lo:hi], zn_err[lo:hi],
                          spectrum_offset=lo + int(kwargs.pop('spectrum_offset', 0)), **kwargs)
-    dev_res = inv.fit_device(None if p0 is None else p0[lo:hi], discard, thin, percentiles, gather_chain, batch_size)
+    # autocorr is passed only when set, so fit_device overrides written for the older signature keep working
+    dev_res = inv.fit_device(None if p0 is None else p0[lo:hi], discard, thin, percentiles, gather_chain, batch_size,
+                             **({'autocorr': True} if autocorr else {}))
     chain = dev_res.pop('chain', None)
     dev_res.pop('log_prob', None)
     if on and world > 1:
@@ -280,15 +283,20 @@ class BatchInversion:
         return max(1, min(65535, int(0.7 * free // per)))
 
     # ------------------------------------------------------------------ fit
-    def fit(self, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), keep_chain=False, batch_size=None):
+    def fit(self, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), keep_chain=False, batch_size=None,
+            autocorr=False):
         """Sample every spectrum and summarise the kept chain on the device.
 
         Returns (and stores in ``self.results``) a dict of host arrays:
         ``percentiles`` (B, len(p), ndim), ``mean`` (B, ndim), ``std`` (B, ndim),
         ``acceptance_fraction`` (B,), ``flags`` (B,), and with ``keep_chain`` the kept
         ``chain`` (B, n_keep, W, ndim) and ``log_prob`` (B, n_keep, W).
+        With ``autocorr=True`` also ``autocorr_time`` (B, ndim): emcee's integrated autocorrelation time of every
+        parameter in steps (``sampler.get_autocorr_time(discard=, thin=, quiet=True)`` of each spectrum), computed on
+        the device from each sub-batch's kept chain before it is dropped; NaN where a walker's kept series is constant.
         """
-        dev_res = self.fit_device(p0, discard, thin, percentiles, keep_chain, batch_size, _chain_to_host=True)
+        dev_res = self.fit_device(p0, discard, thin, percentiles, keep_chain, batch_size, _chain_to_host=True,
+                                  autocorr=autocorr)
         self.percentiles = tuple(float(q) for q in percentiles)
         self.results = {k: (v if isinstance(v, np.ndarray) else v.cpu().numpy()) for k, v in dev_res.items()}
         self._apply_nan_policy(self.results['flags'])
@@ -304,13 +312,14 @@ class BatchInversion:
             import warnings
             warnings.warn(msg, RuntimeWarning)
 
-    def fit_gathered(self, n_total, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), group=None, batch_size=None):
+    def fit_gathered(self, n_total, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), group=None, batch_size=None,
+                     autocorr=False):
         """``fit`` for a shard-local inversion inside a ``torch.distributed`` job: this object holds spectra
         ``[spectrum_offset, spectrum_offset + n_spectra)`` of a survey of ``n_total`` sharded by ``shard_range``; after
         sampling, the summaries of all ranks are all-gathered (one NCCL collective) and the COMPLETE result
         (``n_total`` rows, host arrays) is returned on every rank.  Without a process group it equals ``fit``."""
         import torch.distributed as dist
-        dev_res = self.fit_device(p0, discard, thin, percentiles, False, batch_size)
+        dev_res = self.fit_device(p0, discard, thin, percentiles, False, batch_size, autocorr=autocorr)
         if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
             dev_res = gather_packed(dev_res, int(n_total), dist.get_rank(group), dist.get_world_size(group), group)
         self.percentiles = tuple(float(q) for q in percentiles)
@@ -319,7 +328,7 @@ class BatchInversion:
         return self.results
 
     def fit_device(self, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), keep_chain=False,
-                   batch_size=None, _chain_to_host=False):
+                   batch_size=None, _chain_to_host=False, autocorr=False):
         """Same as ``fit`` but leaves the summaries on the GPU (for the NCCL gather).  With ``keep_chain`` the kept
         chains of all sub-batches stay on the device too (``fit`` moves each sub-batch's chain to the host instead)."""
         B, W, ndim = self.n_spectra, self.nwalkers, self.ndim
@@ -332,6 +341,8 @@ class BatchInversion:
             out = {'percentiles': torch.empty((0, len(percentiles), ndim), **f64), 'mean': torch.empty((0, ndim), **f64),
                    'std': torch.empty((0, ndim), **f64), 'acceptance_fraction': torch.empty((0,), **f64),
                    'flags': torch.empty((0,), dtype=torch.int32, device=self.device)}
+            if autocorr:
+                out['autocorr_time'] = torch.empty((0, ndim), **f64)
             if keep_chain:
                 out['chain'], out['log_prob'] = torch.empty((0, nk, W, ndim), **f64), torch.empty((0, nk, W), **f64)
                 if _chain_to_host:
@@ -342,6 +353,8 @@ class BatchInversion:
         shared_w = self.w.ndim == 1
         w_all = _lib.dev_f64(self.w, self.device) if shared_w else None
         acc = {k: [] for k in ('percentiles', 'mean', 'std', 'acceptance_fraction', 'flags')}
+        if autocorr:
+            acc['autocorr_time'] = []
         if keep_chain:
             acc['chain'], acc['log_prob'] = [], []
         for lo in range(0, B, bs):
@@ -365,6 +378,8 @@ class BatchInversion:
             acc['percentiles'].append(st['pct'])
             acc['mean'].append(st['mean'])
             acc['std'].append(st['std'])
+            if autocorr:                           # emcee's default c = 5; in steps of the run
+                acc['autocorr_time'].append(thin * engine.autocorr_time(res['chain'], 5.0))
             acc['acceptance_fraction'].append(res['accepted'].to(torch.float64).mean(1) / float(self.nsteps))
             acc['flags'].append(res['flags'])
             if keep_chain and _chain_to_host:      # sub-batching stays effective: nothing accumulates on the device
@@ -395,8 +410,7 @@ class BatchInversion:
     def get_autocorr_time(self, c=5, thin=1):
         """Integrated autocorrelation time of every parameter of every spectrum, (B, ndim), from the kept chain of
         the last ``fit(..., keep_chain=True)`` (emcee's estimator; ``thin`` = the thinning that fit used, so the
-        result is in steps).  Evaluated on the GPU in sub-batches."""
-        from .sampler import integrated_time_batch
+        result is in steps).  Evaluated on the GPU in sub-batches by the kernel behind ``fit(..., autocorr=True)``."""
         if self.results is None or 'chain' not in self.results:
             raise AssertionError('get_autocorr_time needs fit(..., keep_chain=True)')
         ch = self.results['chain']
@@ -404,7 +418,7 @@ class BatchInversion:
         step = max(1, int(2 ** 27 // max(1, ch[0].size)))            # ~1 GB of float64 per sub-batch
         for lo in range(0, ch.shape[0], step):
             t = torch.from_numpy(ch[lo:lo + step]).to(self.device)
-            out[lo:lo + step] = integrated_time_batch(t, c=c, thin=thin).cpu().numpy()
+            out[lo:lo + step] = (thin * engine.autocorr_time(t, c)).cpu().numpy()
         return out
 
     def to_csv(self, path, ids=None):

@@ -11,6 +11,7 @@
 #include "launch.cuh"
 #include "stats.cuh"
 #include "model_pct.cuh"
+#include "autocorr.cuh"
 
 namespace bisip {
 
@@ -351,6 +352,28 @@ int bisip_model_percentile(const bisip_model_desc* desc, int n_spectra, int64_t 
   P.st.pct_out = pct_out; P.st.mean_out = nullptr; P.st.std_out = nullptr;
   return launch(model_percentile_kernel, dim3(2 * d.n_freq, n_spectra), smem, (cudaStream_t)stream, "model_percentile", &P,
                 kStatThreads);
+}
+
+int bisip_autocorr_time(const double* data, int n_spectra, int n_keep, int n_walkers, int n_cols, double c,
+                        double* tau_out, void* stream) {
+  if (!data || !tau_out || n_spectra <= 0 || n_keep <= 0 || n_walkers <= 0 || n_cols <= 0)
+    return fail(BISIP_ERR_BAD_ARG, "bisip_autocorr_time: bad argument");
+  if (!std::isfinite(c) || !(c > 0.0)) return fail(BISIP_ERR_BAD_ARG, "bisip_autocorr_time: c must be finite and > 0");
+  if (n_spectra > 65535) return fail(BISIP_ERR_UNSUPPORTED, "bisip_autocorr_time: n_spectra > 65535 per call");
+  DeviceGuard guard(data);
+  AutocorrParams P;
+  P.data = data; P.B = n_spectra; P.n = n_keep; P.W = n_walkers; P.ncol = n_cols; P.c = c; P.tau_out = tau_out;
+  const dim3 grid(n_cols, n_spectra);
+  // the column in shared memory when it fits (the same test as the statistics kernels), else strided global reads
+  const long long nw = (long long)n_keep * n_walkers;
+  const size_t smem = autocorr_smem_bytes(n_keep, n_walkers, true);
+  const int optin = device_smem_optin();
+  if (nw <= 0x7fffffff / 8 && smem + kAcfStaticSmem <= (size_t)optin)
+    return launch(autocorr_kernel<true>, grid, smem, (cudaStream_t)stream, "autocorr_time", &P, kAcfThreads);
+  const size_t gsmem = autocorr_smem_bytes(0, n_walkers, false);
+  if (gsmem + kAcfStaticSmem > (size_t)optin)
+    return fail(BISIP_ERR_UNSUPPORTED, "bisip_autocorr_time: too many walkers for one CTA's shared memory");
+  return launch(autocorr_kernel<false>, grid, gsmem, (cudaStream_t)stream, "autocorr_time", &P, kAcfThreads);
 }
 
 }  // extern "C"

@@ -190,6 +190,23 @@ def column_stats(data, p=None, want_mean=False, want_std=False):
     return out
 
 
+def autocorr_time(chain, c=5.0):
+    """emcee's integrated autocorrelation time of every column: chain (B, n_keep, W, ncol) -> (B, ncol), in steps of
+    the kept chain (``bisip_autocorr_time``; the chain is read in place).  A column with a constant walker or a NaN
+    gives NaN."""
+    lib = _lib.load()
+    _chk_cuda_f64(chain)
+    B, nk, W, ncol = chain.shape
+    dev = chain.device
+    out = torch.empty((B, ncol), dtype=torch.float64, device=dev)
+    for s0 in range(0, B, 65535):                  # one launch per 65,535 spectra (grid y)
+        k = min(65535, B - s0)
+        rc = lib.bisip_autocorr_time(_lib.ptr(chain[s0:s0 + k]), k, nk, W, ncol, float(c), _lib.ptr(out[s0:s0 + k]),
+                                     _lib.stream_ptr(dev))
+        _lib.check(rc, "bisip_autocorr_time")
+    return out
+
+
 def model_percentile(spec, theta, w, p):
     """Percentiles of the forward model over parameter vectors, fused (``bisip_model_percentile``): theta (B, n, ndim),
     w (N,) or (B, N), p percentiles -> (B, len(p), 2, N).  The (n, 2N) model matrix is never materialised.  Returns None

@@ -50,7 +50,8 @@ def load_percentiles_csv(path):
 
 def batch_table(param_names, results, ids=None, percentiles=(2.5, 50, 97.5)):
     """Flatten ``BatchInversion.results`` into (column names, 2-D array): one row per spectrum with
-    id, acceptance fraction, flags, then mean / std / each percentile of every parameter."""
+    id, acceptance fraction, flags, then mean / std / each percentile of every parameter, and — when the results hold
+    ``autocorr_time`` (``fit(..., autocorr=True)``) — one ``<name>_tau`` column per parameter."""
     B = results['mean'].shape[0]
     ids = np.arange(B) if ids is None else np.asarray(ids)
     cols = ['spectrum', 'acceptance_fraction', 'flags']
@@ -62,4 +63,7 @@ def batch_table(param_names, results, ids=None, percentiles=(2.5, 50, 97.5)):
     for k, q in enumerate(percentiles):
         cols += [f'{n}_p{q:g}' for n in param_names]
         blocks.append(results['percentiles'][:, k])
+    if 'autocorr_time' in results:
+        cols += [f'{n}_tau' for n in param_names]
+        blocks.append(results['autocorr_time'])
     return cols, np.concatenate(blocks, axis=1)

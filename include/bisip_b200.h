@@ -21,6 +21,8 @@
  *   bisip_column_stats       <- np.percentile / np.mean / np.std over the flat chain
  *                               (utils.py:35, :53, :69, :85)
  *   bisip_model_percentile   <- utils.get_model_percentile (utils.py:17-35)
+ *   bisip_autocorr_time      <- emcee autocorr.integrated_time, reached through
+ *                               sampler.get_autocorr_time (models.py:154-159)
  *
  * Layouts (all row-major, float64):
  *   theta   [n_spectra][n_theta][ndim]      parameter vectors (order as the reference's
@@ -194,6 +196,21 @@ int bisip_model_percentile(const bisip_model_desc *desc, int n_spectra, int64_t 
                            const double *taus, const double *log_taus, int64_t tau_stride,
                            int n_pct, const int64_t *pct_lo, const double *pct_gamma,
                            double *pct_out, void *stream);
+
+/*
+ * emcee's integrated autocorrelation time (Sokal window, constant c) of every column of
+ * data[n_spectra][n_keep][n_walkers][n_cols], read in place; tau_out[n_spectra][n_cols] in rows of `data`.
+ * Reference: emcee autocorr.integrated_time, reached through sampler.get_autocorr_time (models.py:154-159).
+ * Each walker's series is centred on its own mean, its linear ACF normalised by its lag-0 value, the walkers
+ * averaged, tau(L) = 2 sum_{l<=L} rho(l) - 1, and the result is tau at emcee's automatic window (the first L
+ * with L >= c tau(L)).  In steps of the kept chain: multiply by the thinning for steps of the run.
+ * A column with a constant walker (this includes n_keep == 1) or a NaN gives NaN.  The result of a spectrum
+ * depends on its own column only.  One launch; the lags stop at the window.
+ * BISIP_ERR_BAD_ARG: null pointer, non-positive size, c not finite or <= 0;
+ * BISIP_ERR_UNSUPPORTED: n_spectra > 65535.
+ */
+int bisip_autocorr_time(const double *data, int n_spectra, int n_keep, int n_walkers, int n_cols,
+                        double c, double *tau_out, void *stream);
 
 #ifdef __cplusplus
 }
