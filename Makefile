@@ -14,7 +14,7 @@ UNITS     := api ens_wp_collapsed ens_wp_vec ens_wp_dmma ens_dmma ens_rc ens_umm
 OBJS      := $(UNITS:%=$(CSRC)/%.o)
 
 $(CSRC)/%.o: $(CSRC)/%.cu $(HDRS)
-	$(NVCC) $(NVCCFLAGS) $(EXTRA) -c -o $@ $< 2> $(CSRC)/$*.ptxas || (cat $(CSRC)/$*.ptxas; false)
+	$(NVCC) $(NVCCFLAGS) -c -o $@ $< 2> $(CSRC)/$*.ptxas || (cat $(CSRC)/$*.ptxas; false)
 
 $(LIB): $(OBJS)
 	$(NVCC) $(ARCH) -shared -o $@ $(OBJS)

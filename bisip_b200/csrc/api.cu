@@ -3,8 +3,6 @@
 // plans the launch and holds the statistics entry points.
 #include <atomic>
 #include <cstdio>
-#include <cstring>
-#include <cstdlib>
 #include <cmath>
 #include <string>
 
@@ -29,6 +27,10 @@ void count_launches(int n) { g_launches.fetch_add(n); }
 using namespace bisip;
 
 namespace {
+
+// Start delay of the second co-resident CTA of ensemble_kernel (sampler.cuh, stagger_start): a quarter of one
+// ensemble step, estimated from the tile count.
+constexpr unsigned long long kStaggerNs = 6000ull;
 
 // The kernels must run on the device that owns the caller's buffers, whatever device is current in the calling
 // thread (one host thread may drive several GPUs): the entry points switch to the device of their primary pointer
@@ -213,40 +215,31 @@ int bisip_ensemble_run(const bisip_model_desc* desc, int n_spectra, int n_walker
     P.a_pow2 = (frexp(a, &ex) == 0.5) ? 1 : 0;
     P.inv_a = 1.0 / a;
   }
-  {
-    // developer knob; default = a quarter of one ensemble step, estimated from the tile count
-    const char* e = getenv("BISIP_STAGGER_NS");
-    P.stagger_ns = e ? strtoull(e, nullptr, 10) : 6000ull;
-  }
+  P.stagger_ns = kStaggerNs;
   if (flags) BISIP_CUDA(cudaMemsetAsync(flags, 0, sizeof(int32_t) * (size_t)n_spectra, st));
   const int rp = sampler_rows_pad(n_walkers);
   size_t smem = sampler_smem_bytes(n_walkers, desc->ndim);
   dim3 grid(n_spectra);
-  // Warp-private sampler (sampler_wp.cuh) for the evaluators that have a warp-level form, up to 256 walkers.
-  // BISIP_SAMPLER=classic forces the block-synchronous kernel (developer comparison; both follow the same stream).
-  {
-    const char* e = getenv("BISIP_SAMPLER");
-    const bool classic = e && !strcmp(e, "classic");
-    const bool big_poly = desc->model == BISIP_MODEL_DECOMP && desc->n_coef > 8;     // FP64 on the collapsed tiles only
-    if (big_poly && n_walkers > 256)
-      return fail(BISIP_ERR_UNSUPPORTED, "Decomp poly_deg > 7 is sampled by the warp-private kernel: at most 256 walkers");
-    if ((!classic || big_poly) && n_walkers <= 256) {
-      if (desc->model == BISIP_MODEL_DECOMP && (desc->precision == BISIP_PREC_FP64_COLLAPSED || big_poly))
-        return launch_ens_wp_collapsed(P, grid, st);
-      if (desc->model == BISIP_MODEL_DECOMP && desc->precision == BISIP_PREC_FP64 && desc->n_tau > 32 && desc->n_tau <= 64)
-        return launch_ens_wp_dmma(P, grid, st);
-      // measured (profiles/r02_wp_sweep.md, r02c_vec_analysis.md): warp-private wins by 1.2-2x for <= 64 walkers or short
-      // spectra and for 1-mode Cole-Cole everywhere; for Dias / Shin / 2-mode Cole-Cole with > 64 walkers and > 32
-      // frequencies the block-synchronous kernel is 2-7 % faster (its serial phases run on full warps; the long frequency
-      // loop dominates either way).  BISIP_SAMPLER=wp forces the warp-private kernel there (developer comparison).
-      const bool force_wp = e && !strcmp(e, "wp");
-      const bool long_vec = n_walkers > 64 && desc->n_freq > 32 && !force_wp;
-      const bool wp_vec = desc->model == BISIP_MODEL_DIAS || desc->model == BISIP_MODEL_SHIN
-                              ? !long_vec
-                              : desc->model == BISIP_MODEL_COLECOLE && (desc->n_modes == 1 || (desc->n_modes == 2 && !long_vec));
-      if (wp_vec)
-        return launch_ens_wp_vec(P, grid, st);
-    }
+  // Warp-private sampler (sampler_wp.cuh) for the evaluators that have a warp-level form, up to 256 walkers; both
+  // kernels follow the same stream.
+  const bool big_poly = desc->model == BISIP_MODEL_DECOMP && desc->n_coef > 8;     // FP64 on the collapsed tiles only
+  if (big_poly && n_walkers > 256)
+    return fail(BISIP_ERR_UNSUPPORTED, "Decomp poly_deg > 7 is sampled by the warp-private kernel: at most 256 walkers");
+  if (n_walkers <= 256) {
+    if (desc->model == BISIP_MODEL_DECOMP && (desc->precision == BISIP_PREC_FP64_COLLAPSED || big_poly))
+      return launch_ens_wp_collapsed(P, grid, st);
+    if (desc->model == BISIP_MODEL_DECOMP && desc->precision == BISIP_PREC_FP64 && desc->n_tau > 32 && desc->n_tau <= 64)
+      return launch_ens_wp_dmma(P, grid, st);
+    // measured (profiles/r02_wp_sweep.md, r02c_vec_analysis.md): warp-private wins by 1.2-2x for <= 64 walkers or short
+    // spectra and for 1-mode Cole-Cole everywhere; for Dias / Shin / 2-mode Cole-Cole with > 64 walkers and > 32
+    // frequencies the block-synchronous kernel is 2-7 % faster (its serial phases run on full warps; the long frequency
+    // loop dominates either way).
+    const bool long_vec = n_walkers > 64 && desc->n_freq > 32;
+    const bool wp_vec = desc->model == BISIP_MODEL_DIAS || desc->model == BISIP_MODEL_SHIN
+                            ? !long_vec
+                            : desc->model == BISIP_MODEL_COLECOLE && (desc->n_modes == 1 || (desc->n_modes == 2 && !long_vec));
+    if (wp_vec)
+      return launch_ens_wp_vec(P, grid, st);
   }
   switch (desc->model) {
     case BISIP_MODEL_COLECOLE:

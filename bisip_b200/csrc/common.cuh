@@ -10,10 +10,7 @@
 
 namespace bisip {
 
-#ifndef BISIP_THREADS
-#define BISIP_THREADS 256
-#endif
-constexpr int kThreads = BISIP_THREADS;   // CTA size of every hot-path kernel (developer sweeps: -DBISIP_THREADS=128)
+constexpr int kThreads = 256;   // CTA size of every hot-path kernel
 constexpr int kWarps = kThreads / 32;
 
 // ---------------------------------------------------------------- Philox4x32-10

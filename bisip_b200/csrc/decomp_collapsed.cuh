@@ -109,10 +109,7 @@ __device__ inline void decomp_c_init(DecompCSmem& s, const DecompCShape& sh, dou
 // Rows (proposals) per thread of the register tile: every column record read from shared memory then feeds
 // kCRows rows, which divides the LDS.128 traffic per FMA by kCRows (the broadcast loads, not the FP64 pipe, bound
 // the one-row version: 4 LDS.128 per 7.5 DFMA).  Used when there are at least 32*kCRows rows; else one row per thread.
-#ifndef BISIP_COLLAPSED_RPT
-#define BISIP_COLLAPSED_RPT 2
-#endif
-constexpr int kCRows = BISIP_COLLAPSED_RPT;
+constexpr int kCRows = 2;
 
 // Work split of an evaluation, a function of the largest number of rows the CTA evaluates (`rows_cap`) only:
 // thread-rows (rpt proposals each) padded to a power of two >= 32 so that a warp works on ONE group, the N frequencies

@@ -196,10 +196,7 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* v) {
 
 // suspend-time hint of mbarrier.try_wait: the waiting warps sleep instead of re-issuing the poll (the polls were 5 % of
 // all issued instructions of the sampler kernel)
-#ifndef BISIP_UMMA_WAIT_HINT
-#define BISIP_UMMA_WAIT_HINT 2000
-#endif
-constexpr uint32_t kUmmaWaitHintNs = BISIP_UMMA_WAIT_HINT;
+constexpr uint32_t kUmmaWaitHintNs = 2000;
 __device__ __forceinline__ void mbar_wait(uint32_t baddr, uint32_t parity) {
   uint32_t done = 0;
   while (!done) {
@@ -222,31 +219,21 @@ __device__ __forceinline__ void split3_tf32(double x, uint32_t& hi, uint32_t& mi
   lo = tf32_rn((r1 - __uint_as_float(mid)) + xl);
 }
 // two-way split of an FP32 value (22 bits).  The re-pack of M runs this on 64 values per proposal and half-step: it was
-// 20 % of all instructions of the 3xTF32 sampler kernel, most of them integer (half rate on B200).
-//   BISIP_UMMA_SPLIT2 = 0  hi = rn(x), lo = rn(x - hi)                      5 instructions (round 1)
-//                       1  hi = rn(x), lo = x - hi left in FP32            3: the tensor core ignores the low 13 mantissa bits
-//                          (default)                                          of a tf32 operand, i.e. truncates lo itself
-//                       2  hi = x with the low 13 bits cleared, lo = x - hi  2: truncation on both levels
+// 20 % of all instructions of the 3xTF32 sampler kernel, most of them integer (half rate on B200).  Three splits were
+// compared; split2_tf32 is variant 1:
+//   0  hi = rn(x), lo = rn(x - hi)                      5 instructions (round 1)
+//   1  hi = rn(x), lo = x - hi left in FP32            3: the tensor core ignores the low 13 mantissa bits of a tf32
+//                                                         operand, i.e. truncates lo itself
+//   2  hi = x with the low 13 bits cleared, lo = x - hi  2: truncation on both levels
 // Measured (profiles/r02d_barriers.md): forward error of 3xTF32 8.3e-8 / 8.4e-8 / 1.2e-7, sampler 6.53e9 / 6.62e9 / 6.58e9
 // evals/s for 0 / 1 / 2; variant 2 also truncates the only plane of plain TF32 (5.6e-5 -> 1.9e-4), so 1 it is.
-#ifndef BISIP_UMMA_SPLIT2
-#define BISIP_UMMA_SPLIT2 1
-#endif
 __device__ __forceinline__ void split2_tf32_rn(float x, uint32_t& hi, uint32_t& lo) {      // init-time planes: always rounded
   hi = tf32_rn(x);
   lo = tf32_rn(x - __uint_as_float(hi));
 }
 __device__ __forceinline__ void split2_tf32(float x, uint32_t& hi, uint32_t& lo) {
-#if BISIP_UMMA_SPLIT2 == 2
-  hi = __float_as_uint(x) & 0xffffe000u;
-  lo = __float_as_uint(x - __uint_as_float(hi));
-#elif BISIP_UMMA_SPLIT2 == 1
   hi = tf32_rn(x);
   lo = __float_as_uint(x - __uint_as_float(hi));
-#else
-  hi = tf32_rn(x);
-  lo = tf32_rn(x - __uint_as_float(hi));
-#endif
 }
 
 // Per-spectrum constants; allocates tensor memory.  All threads; ends with __syncthreads().

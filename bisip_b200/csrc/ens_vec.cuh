@@ -8,11 +8,7 @@
 
 namespace bisip {
 
-#ifdef BISIP_VEC_MINB
-constexpr int kMinBVec = BISIP_VEC_MINB;
-#else
 constexpr int kMinBVec = 4;      // 256-thread CTAs, 64 registers
-#endif
 constexpr int kVecSmallW = 128;  // walkers up to which the 128-thread variant is used
 
 // launch ensemble_kernel<VecEvaluator<Row>> in the shape picked for W walkers; MB128 = CTAs/SM of the

@@ -3,16 +3,12 @@
 
 namespace bisip {
 
-#ifndef BISIP_WP_COLLAPSED_REGS
-#define BISIP_WP_COLLAPSED_REGS 64
-#endif
-
 int launch_ens_wp_collapsed(const EnsembleParams& P, dim3 grid, cudaStream_t st) {
   const int KS = (P.d.n_coef + 2 + 7) / 8;
   const size_t other = wp_smem_bytes(P.W, P.d.ndim);
   switch (KS) {
-    case 1: return launch_wp<CollapsedMmaEvaluator<1>, BISIP_WP_COLLAPSED_REGS>(P, grid, other + CollapsedMmaEvaluator<1>::smem_doubles(P.d) * 8, st, "ensemble_wp_decomp_collapsed");
-    case 2: return launch_wp<CollapsedMmaEvaluator<2>, BISIP_WP_COLLAPSED_REGS>(P, grid, other + CollapsedMmaEvaluator<2>::smem_doubles(P.d) * 8, st, "ensemble_wp_decomp_collapsed");
+    case 1: return launch_wp<CollapsedMmaEvaluator<1>, 64>(P, grid, other + CollapsedMmaEvaluator<1>::smem_doubles(P.d) * 8, st, "ensemble_wp_decomp_collapsed");
+    case 2: return launch_wp<CollapsedMmaEvaluator<2>, 64>(P, grid, other + CollapsedMmaEvaluator<2>::smem_doubles(P.d) * 8, st, "ensemble_wp_decomp_collapsed");
     default: return launch_wp<CollapsedMmaEvaluator<4>, 80>(P, grid, other + CollapsedMmaEvaluator<4>::smem_doubles(P.d) * 8, st, "ensemble_wp_decomp_collapsed");
   }
 }

@@ -823,23 +823,11 @@ __global__ void __launch_bounds__(NT, MINB) ensemble_kernel(const EnsembleParams
   // doubled one included (same-box A/B, profiles/r02d_barriers.md: Dias, 128 walkers, 7.01e9 vs 6.95e9 on full waves, 6.30e9
   // vs 6.06e9 on the 1,024 spectra of BASELINE config 3; Shin is 0.6 % faster with the short one): their barriers are free
   // (other CTAs fill them) and apparently keep the co-resident CTAs out of phase.
-#ifdef BISIP_LEGACY_RANK
-  constexpr bool kLegacyRank = BISIP_LEGACY_RANK != 0;
-#else
   constexpr bool kLegacyRank = Eval::kLegacyRank;
-#endif
-#ifdef BISIP_PAIR_PROPOSE
-  constexpr bool kPairPropose = BISIP_PAIR_PROPOSE != 0;
-#else
   constexpr bool kPairPropose = Eval::kClustered;   // same-box A/B (profiles/r02d_barriers.md): clustered evaluators +0.4-1 %, TF32 tcgen05 -2 %
-#endif
   // bin slots of the key ranking inside the second accept phase (one CTA barrier less per step) or in a phase of their
   // own: +-1-2 % either way depending on the evaluator and the CTA size (profiles/r02d_barriers.md)
-#ifdef BISIP_RANK_IN_ACCEPT
-  constexpr bool kRankInAccept = BISIP_RANK_IN_ACCEPT != 0;
-#else
   constexpr bool kRankInAccept = Eval::kRankInAccept && (NT == 128 || Eval::kClustered || !Eval::kNeedsPrepare);
-#endif
   PHASE_DECL
   for (int it = 0; it < P.nsteps; ++it) {
     const uint32_t t = (uint32_t)(P.step0 + it);

@@ -48,6 +48,9 @@ SHAPES = [
     ('decomp', 7, 18, 50, dict(poly_deg=2, n_tau=9, c_exp=0.5)), # one k chunk, 2N = 14 columns
     ('decomp', 64, 40, 20, dict(poly_deg=4, n_tau=65)),          # smallest clustered (n_tau > 64) case
     ('decomp', 31, 258, 6, dict(poly_deg=5, n_tau=200, c_exp=0.7)),
+    ('colecole', 33, 260, 8, dict(n_modes=1)),     # 1 mode beyond the warp-private kernel's 256 walkers
+    ('colecole', 40, 140, 12, dict(n_modes=2)),    # 2 modes, > 128 walkers, > 32 frequencies: 256-thread variant
+    ('decomp', 40, 270, 6, dict(poly_deg=3, n_tau=40)),          # 33-48 taus beyond the warp-private kernel's 256 walkers
 ]
 
 
