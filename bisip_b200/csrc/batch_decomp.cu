@@ -1,179 +1,13 @@
 // Batched forward / log-probability of the polynomial decomposition (same evaluators as the sampler).
-// grid (chunks, B): CTA (c, b) handles theta rows [c*kRows, ...) of spectrum b, striding by gridDim.x.
-#include "launch.cuh"
+#include "batch.cuh"
 
 namespace bisip {
 
-template <int KC, bool WANT_Z>
-__global__ void __launch_bounds__(kThreads) decomp_batch_kernel(const BatchParams P) {
-  extern __shared__ __align__(16) double smem[];
-  const int b = blockIdx.y, ndim = P.d.ndim, N = P.d.n_freq;
-  DecompShape sh(P.d.n_freq, P.d.n_tau, P.d.n_coef);
-  DecompSmem s;
-  double* p = decomp_carve(s, smem, sh, kRows);
-  double* prop = p; p += kRows * ndim;
-  double* chi = p; p += kRows;
-  double* bnd = p; p += 2 * ndim;
-  double* red = p;
-  if (!WANT_Z) for (int i = threadIdx.x; i < 2 * ndim; i += kThreads) bnd[i] = P.bounds[i];
-  decomp_init(s, sh, P.d.c_exp, P.w + (size_t)b * P.w_stride, P.taus + (size_t)b * P.tau_stride,
-              P.log_taus + (size_t)b * P.tau_stride * P.d.n_coef,
-              WANT_Z ? nullptr : P.y + (size_t)b * 2 * N, WANT_Z ? nullptr : P.yerr + (size_t)b * 2 * N, red);
-  for (int r0 = blockIdx.x * kRows; r0 < P.n_theta; r0 += gridDim.x * kRows) {
-    const int n = min(kRows, P.n_theta - r0);
-    const double* th = P.theta + ((size_t)b * P.n_theta + r0) * ndim;
-    for (int i = threadIdx.x; i < kRows * ndim; i += kThreads) prop[i] = (i < n * ndim) ? th[i] : 0.0;
-    __syncthreads();
-    if (WANT_Z) {
-      decomp_eval_Z<KC>(s, sh, prop, ndim, n, P.Z + ((size_t)b * P.n_theta + r0) * 2 * N);
-    } else {
-      NoSide ns;
-      decomp_eval_chi<KC>(s, sh, prop, ndim, n, kRows, chi, ns);
-      __syncthreads();
-      for (int q = threadIdx.x; q < n; q += kThreads)
-        P.lp[(size_t)b * P.n_theta + r0 + q] =
-            in_bounds(prop + q * ndim, bnd, ndim) ? -0.5 * (chi[q] + s.llconst) : neg_inf();
-    }
-    __syncthreads();
-  }
-}
-
-// Collapsed decomposition (decomp_collapsed.cuh): same grid as decomp_batch_kernel.
-template <bool WANT_Z>
-__global__ void __launch_bounds__(kThreads) decomp_c_batch_kernel(const BatchParams P) {
-  extern __shared__ __align__(16) double smem[];
-  const int b = blockIdx.y, ndim = P.d.ndim, N = P.d.n_freq;
-  DecompCShape sh(P.d.n_freq, P.d.n_tau, P.d.n_coef);
-  DecompCSmem s;
-  double* p = decomp_c_carve(s, smem, sh, kRows);
-  double* prop = p; p += kRows * ndim;
-  double* chi = p; p += kRows;
-  double* bnd = p; p += 2 * ndim;
-  double* red = p;
-  if (!WANT_Z) for (int i = threadIdx.x; i < 2 * ndim; i += kThreads) bnd[i] = P.bounds[i];
-  decomp_c_init(s, sh, P.d.c_exp, P.w + (size_t)b * P.w_stride, P.taus + (size_t)b * P.tau_stride,
-                P.log_taus + (size_t)b * P.tau_stride * P.d.n_coef,
-                WANT_Z ? nullptr : P.y + (size_t)b * 2 * N, WANT_Z ? nullptr : P.yerr + (size_t)b * 2 * N, red);
-  for (int r0 = blockIdx.x * kRows; r0 < P.n_theta; r0 += gridDim.x * kRows) {
-    const int n = min(kRows, P.n_theta - r0);
-    const double* th = P.theta + ((size_t)b * P.n_theta + r0) * ndim;
-    for (int i = threadIdx.x; i < kRows * ndim; i += kThreads) prop[i] = (i < n * ndim) ? th[i] : 0.0;
-    __syncthreads();
-    if (WANT_Z) {
-      decomp_c_eval_Z(s, sh, prop, ndim, n, P.Z + ((size_t)b * P.n_theta + r0) * 2 * N);
-    } else {
-      decomp_c_eval_chi(s, sh, prop, ndim, n, kRows, chi);
-      __syncthreads();
-      for (int q = threadIdx.x; q < n; q += kThreads)
-        P.lp[(size_t)b * P.n_theta + r0 + q] =
-            in_bounds(prop + q * ndim, bnd, ndim) ? -0.5 * (chi[q] + s.llconst) : neg_inf();
-    }
-    __syncthreads();
-  }
-}
-
-// uniform access to the three clustered evaluators for the batch kernel
-template <int PREC> struct RcOps;
-template <> struct RcOps<0> {
-  using Smem = DecompRCSmem;
-  static __device__ double* carve(Smem& s, double* b, const DecompRCShape& sh, int rp) { return decomp_rc_carve(s, b, sh, rp); }
-  template <class... A> static __device__ void init(A&&... a) { decomp_rc_init(a...); }
-  template <class... A> static __device__ void chi(A&&... a) { decomp_rc_eval_chi(a...); }
-  template <class... A> static __device__ void Z(A&&... a) { decomp_rc_eval_Z(a...); }
-};
-template <> struct RcOps<1> {
-  using Smem = DecompTF32Smem;
-  static __device__ double* carve(Smem& s, double* b, const DecompRCShape& sh, int rp) { return decomp_tf32_carve<1>(s, b, sh, rp); }
-  template <class... A> static __device__ void init(A&&... a) { decomp_tf32_init<1>(a...); }
-  template <class... A> static __device__ void chi(A&&... a) { decomp_tf32_eval_chi<1>(a...); }
-  template <class... A> static __device__ void Z(A&&... a) { decomp_tf32_eval_Z<1>(a...); }
-};
-template <> struct RcOps<3> {
-  using Smem = DecompTF32Smem;
-  static __device__ double* carve(Smem& s, double* b, const DecompRCShape& sh, int rp) { return decomp_tf32_carve<3>(s, b, sh, rp); }
-  template <class... A> static __device__ void init(A&&... a) { decomp_tf32_init<3>(a...); }
-  template <class... A> static __device__ void chi(A&&... a) { decomp_tf32_eval_chi<3>(a...); }
-  template <class... A> static __device__ void Z(A&&... a) { decomp_tf32_eval_Z<3>(a...); }
-};
-
-// Batched forward / log-probability for large tau grids: grid (chunks*CS, B), cluster (CS,1,1).
-template <int PREC, bool WANT_Z>
-__global__ void __launch_bounds__(kThreads) decomp_rc_batch_kernel(const BatchParams P) {
-  using Ops = RcOps<PREC>;
-  extern __shared__ __align__(16) double smem[];
-  cg::cluster_group cluster = cg::this_cluster();
-  const int cs = (int)cluster.num_blocks(), crank = (int)cluster.block_rank();
-  const int b = blockIdx.y, ndim = P.d.ndim, N = P.d.n_freq;
-  const int chunk0 = blockIdx.x / cs, nchunks = gridDim.x / cs;
-  DecompRCShape sh(P.d.n_freq, P.d.n_tau, P.d.n_coef, cs, crank);
-  typename Ops::Smem s;
-  double* p = Ops::carve(s, smem, sh, kRows);
-  double* prop = p; p += kRows * ndim;
-  double* chi = p; p += kRows;
-  double* bnd = p; p += 2 * ndim;
-  double* red = p;
-  if (!WANT_Z) for (int i = threadIdx.x; i < 2 * ndim; i += kThreads) bnd[i] = P.bounds[i];
-  Ops::init(s, sh, P.d.c_exp, P.w + (size_t)b * P.w_stride, P.taus + (size_t)b * P.tau_stride,
-                 P.log_taus + (size_t)b * P.tau_stride * P.d.n_coef,
-                 WANT_Z ? nullptr : P.y + (size_t)b * 2 * N, WANT_Z ? nullptr : P.yerr + (size_t)b * 2 * N, red);
-  for (int r0 = chunk0 * kRows; r0 < P.n_theta; r0 += nchunks * kRows) {
-    const int n = min(kRows, P.n_theta - r0);
-    const double* th = P.theta + ((size_t)b * P.n_theta + r0) * ndim;
-    for (int i = threadIdx.x; i < kRows * ndim; i += kThreads) prop[i] = (i < n * ndim) ? th[i] : 0.0;
-    __syncthreads();
-    if (WANT_Z) {
-      Ops::Z(s, sh, prop, ndim, n, P.Z + ((size_t)b * P.n_theta + r0) * 2 * N);
-    } else {
-      const int rows_cap = kRows;
-      Ops::chi(s, sh, prop, ndim, n, rows_cap, chi);
-      __syncthreads();
-      if (crank == 0)
-        for (int q = threadIdx.x; q < n; q += kThreads)
-          P.lp[(size_t)b * P.n_theta + r0 + q] =
-              in_bounds(prop + q * ndim, bnd, ndim) ? -0.5 * (chi[q] + s.llconst) : neg_inf();
-    }
-    __syncthreads();
-  }
-  if (cs > 1) cluster.sync();
-}
-
-// Batched forward / log-probability on the tcgen05 path: grid (chunks, B), 128 theta rows per tile.
-template <int PREC, bool WANT_Z>
-__global__ void __launch_bounds__(kThreads) decomp_umma_batch_kernel(const BatchParams P) {
-  extern __shared__ __align__(16) double smem[];
-  const int b = blockIdx.y, ndim = P.d.ndim, N = P.d.n_freq;
-  DecompUmmaShape sh(P.d.n_freq, P.d.n_tau, P.d.n_coef);
-  DecompUmmaSmem s;
-  double* p = decomp_umma_carve<PREC>(s, smem, sh);
-  double* prop = p; p += kRows * ndim;
-  double* chi = p; p += kRows;
-  double* bnd = p; p += 2 * ndim;
-  double* red = p;
-  if (!WANT_Z) for (int i = threadIdx.x; i < 2 * ndim; i += kThreads) bnd[i] = P.bounds[i];
-  decomp_umma_init<PREC>(s, sh, P.d.c_exp, P.w + (size_t)b * P.w_stride, P.taus + (size_t)b * P.tau_stride,
-                         P.log_taus + (size_t)b * P.tau_stride * P.d.n_coef,
-                         WANT_Z ? nullptr : P.y + (size_t)b * 2 * N, WANT_Z ? nullptr : P.yerr + (size_t)b * 2 * N, red);
-  for (int r0 = blockIdx.x * kRows; r0 < P.n_theta; r0 += gridDim.x * kRows) {
-    const int n = min(kRows, P.n_theta - r0);
-    const double* th = P.theta + ((size_t)b * P.n_theta + r0) * ndim;
-    for (int i = threadIdx.x; i < kRows * ndim; i += kThreads) prop[i] = (i < n * ndim) ? th[i] : 0.0;
-    __syncthreads();
-    decomp_umma_eval<PREC, WANT_Z>(s, sh, prop, ndim, n, chi,
-                                   WANT_Z ? P.Z + ((size_t)b * P.n_theta + r0) * 2 * N : nullptr);
-    __syncthreads();
-    if (!WANT_Z)
-      for (int q = threadIdx.x; q < n; q += kThreads)
-        P.lp[(size_t)b * P.n_theta + r0 + q] =
-            in_bounds(prop + q * ndim, bnd, ndim) ? -0.5 * (chi[q] + s.llconst) : neg_inf();
-    __syncthreads();
-  }
-  decomp_umma_release(s, sh);
-}
-
-// More than 8 polynomial coefficients (poly_deg > 7): none of the tile shapes above holds the stage-1 operand.  The
+// More than 8 polynomial coefficients (poly_deg > 7): none of the evaluators' tile shapes holds the stage-1 operand.  The
 // forward is evaluated in its collapsed FP64 form Z_c = R0 (delta_c - sum_i a_i G_ic), G = L K accumulated once per CTA
 // in compensated (Dot2) arithmetic like decomp_c_init — plain loops, any n_coef <= 30: this is the API path of
-// forward() / _log_probability() for large polynomials, not a sampled path.  Same grid as decomp_batch_kernel.
+// forward() / _log_probability() for large polynomials, not a sampled path.  Grid (rows, B): CTA (r, b) handles theta
+// rows r, r + gridDim.x, ... of spectrum b.
 constexpr int kBigD = 30;
 template <bool WANT_Z>
 __global__ void __launch_bounds__(kThreads) decomp_big_batch_kernel(const BatchParams P) {
@@ -201,22 +35,7 @@ __global__ void __launch_bounds__(kThreads) decomp_big_batch_kernel(const BatchP
     const int c = idx / D, i = idx - c * D;
     const int j = c < N ? c : c - N;
     const double is = WANT_Z ? 1.0 : 1.0 / yerr[c];
-    const double* lt = lts + (size_t)i * S;
-    double sum = 0.0, comp = 0.0;
-    for (int k = 0; k < S; ++k) {
-      double kre, kim;
-      debye_kernel_term(w[j], taus[k], P.d.c_exp, cs, sn, kre, kim);
-      const double kv = (c < N ? kre : kim) * is;
-      const double l = lt[k];
-      const double p = __dmul_rn(l, kv);
-      const double pe = __fma_rn(l, kv, -p);
-      const double t = __dadd_rn(sum, p);
-      const double bb = __dsub_rn(t, sum);
-      const double se = __dadd_rn(__dsub_rn(sum, __dsub_rn(t, bb)), __dsub_rn(p, bb));
-      sum = t;
-      comp = __dadd_rn(comp, __dadd_rn(se, pe));
-    }
-    G[idx] = sum + comp;
+    G[idx] = dot2_lk(lts + (size_t)i * S, taus, S, w[j], P.d.c_exp, cs, sn, c >= N, is);
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) csum += __shfl_xor_sync(0xffffffffu, csum, o);
@@ -258,56 +77,37 @@ __global__ void __launch_bounds__(kThreads) decomp_big_batch_kernel(const BatchP
 
 template <bool WANT_Z>
 static int run_batch_decomp_t(const BatchParams& P, cudaStream_t st) {
-  const size_t other = batch_other_bytes(P.d);
   if (P.d.n_coef > 8) {
     if (P.d.n_coef > kBigD) return fail(BISIP_ERR_UNSUPPORTED, "Decomp poly_deg > 29 not supported");
     const size_t smem = ((size_t)2 * P.d.n_freq * (P.d.n_coef + 2)) * 8;
-    const int rows = max(1, min(P.n_theta, (148 * 8) / max(1, P.B)));
+    const int rows = max(1, min(P.n_theta, device_sm_count() * 8 / max(1, P.B)));
     return launch(decomp_big_batch_kernel<WANT_Z>, dim3(rows, P.B), smem, st, "decomp_big_batch", &P);
   }
-  {
-    const UmmaPlan up = plan_umma(P.d, other, kRows);
-    if (up.ok) {
-      int chunks = ceil_div(P.n_theta, kRows);
-      const int cap = max(1, (148 * 2) / max(1, P.B));
-      if (chunks > cap) chunks = cap;
-      const dim3 g(chunks, P.B);
-      if (prec_planes(P.d.precision) == 3)
-        return launch(decomp_umma_batch_kernel<3, WANT_Z>, g, up.smem, st, "decomp_umma_3xtf32_batch", &P);
-      return launch(decomp_umma_batch_kernel<1, WANT_Z>, g, up.smem, st, "decomp_umma_tf32_batch", &P);
-    }
+  const size_t other = batch_other_bytes(P.d);
+  const UmmaPlan up = plan_umma(P.d, other, kRows);
+  if (up.ok) {
+    if (prec_planes(P.d.precision) == 3)
+      return launch_batch<DecompUmmaEvaluator<3>, WANT_Z>(P, 2, up.smem, st, "decomp_umma_3xtf32_batch");
+    return launch_batch<DecompUmmaEvaluator<1>, WANT_Z>(P, 2, up.smem, st, "decomp_umma_tf32_batch");
   }
-  if (P.d.precision == BISIP_PREC_FP64_COLLAPSED) {
-    const size_t smem = other + decomp_c_smem_doubles(DecompCShape(P.d.n_freq, P.d.n_tau, P.d.n_coef), kRows) * 8;
-    int chunks = ceil_div(P.n_theta, kRows);
-    const int cap = max(1, (148 * 4) / max(1, P.B));
-    if (chunks > cap) chunks = cap;
-    return launch(decomp_c_batch_kernel<WANT_Z>, dim3(chunks, P.B), smem, st, "decomp_collapsed_batch", &P);
-  }
+  if (P.d.precision == BISIP_PREC_FP64_COLLAPSED)
+    return launch_batch<DecompCollapsedEvaluator, WANT_Z>(P, 4, batch_smem<DecompCollapsedEvaluator>(P.d), st,
+                                                          "decomp_collapsed_batch");
   if (use_rc(P.d)) {
     RcPlan plan;
     if (int rc = plan_rc(P.d, other, kRows, &plan)) return rc;
-    int chunks = ceil_div(P.n_theta, kRows);
-    const int cap = max(1, (148 * 2) / max(1, P.B * plan.cs));
-    if (chunks > cap) chunks = cap;
-    const dim3 g(chunks * plan.cs, P.B);
     switch (prec_planes(P.d.precision)) {
-      case 1: return launch_cluster(decomp_rc_batch_kernel<1, WANT_Z>, g, plan.cs, plan.smem, st, "decomp_tf32_batch", &P);
-      case 3: return launch_cluster(decomp_rc_batch_kernel<3, WANT_Z>, g, plan.cs, plan.smem, st, "decomp_3xtf32_batch", &P);
-      default: return launch_cluster(decomp_rc_batch_kernel<0, WANT_Z>, g, plan.cs, plan.smem, st, "decomp_rc_batch", &P);
+      case 1: return launch_batch<DecompTF32Evaluator<1>, WANT_Z>(P, 2, plan.smem, st, "decomp_tf32_batch", plan.cs);
+      case 3: return launch_batch<DecompTF32Evaluator<3>, WANT_Z>(P, 2, plan.smem, st, "decomp_3xtf32_batch", plan.cs);
+      default: return launch_batch<DecompRCEvaluator, WANT_Z>(P, 2, plan.smem, st, "decomp_rc_batch", plan.cs);
     }
   }
-  const size_t smem = other + decomp_smem_doubles(DecompShape(P.d.n_freq, P.d.n_tau, P.d.n_coef), kRows) * 8;
-  int chunks = ceil_div(P.n_theta, kRows);
-  const int cap = max(1, (148 * 8) / max(1, P.B));   // enough CTAs to fill the chip, no more
-  if (chunks > cap) chunks = cap;
-  const dim3 grid(chunks, P.B);
-  const int KC = ceil_div(P.d.n_tau, 16);
-  switch (KC) {
-    case 1: return launch(decomp_batch_kernel<1, WANT_Z>, grid, smem, st, "decomp_batch", &P);
-    case 2: return launch(decomp_batch_kernel<2, WANT_Z>, grid, smem, st, "decomp_batch", &P);
-    case 3: return launch(decomp_batch_kernel<3, WANT_Z>, grid, smem, st, "decomp_batch", &P);
-    default: return launch(decomp_batch_kernel<4, WANT_Z>, grid, smem, st, "decomp_batch", &P);
+  const size_t smem = batch_smem<DecompEvaluator<1>>(P.d);     // the same for every KC
+  switch (ceil_div(P.d.n_tau, 16)) {
+    case 1: return launch_batch<DecompEvaluator<1>, WANT_Z>(P, 8, smem, st, "decomp_batch");
+    case 2: return launch_batch<DecompEvaluator<2>, WANT_Z>(P, 8, smem, st, "decomp_batch");
+    case 3: return launch_batch<DecompEvaluator<3>, WANT_Z>(P, 8, smem, st, "decomp_batch");
+    default: return launch_batch<DecompEvaluator<4>, WANT_Z>(P, 8, smem, st, "decomp_batch");
   }
 }
 

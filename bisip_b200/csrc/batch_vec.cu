@@ -1,61 +1,28 @@
 // Batched forward / log-probability of the Cole-Cole / Dias / Shin models (same evaluators as the sampler).
-#include "launch.cuh"
+#include "batch.cuh"
 
 namespace bisip {
 
 template <class Row, bool WANT_Z>
-__global__ void __launch_bounds__(kThreads) vec_batch_kernel(const BatchParams P) {
-  extern __shared__ __align__(16) double smem[];
-  const int b = blockIdx.y, ndim = P.d.ndim, N = P.d.n_freq;
-  VecSmem s;
-  double* p = vec_carve(s, smem, N, kRows, Row::kRC);
-  double* prop = p; p += kRows * ndim;
-  double* chi = p; p += kRows;
-  double* bnd = p; p += 2 * ndim;
-  double* red = p;
-  if (!WANT_Z) for (int i = threadIdx.x; i < 2 * ndim; i += kThreads) bnd[i] = P.bounds[i];
-  vec_init(s, N, P.w + (size_t)b * P.w_stride, WANT_Z ? nullptr : P.y + (size_t)b * 2 * N,
-           WANT_Z ? nullptr : P.yerr + (size_t)b * 2 * N, red);
-  for (int r0 = blockIdx.x * kRows; r0 < P.n_theta; r0 += gridDim.x * kRows) {
-    const int n = min(kRows, P.n_theta - r0);
-    const double* th = P.theta + ((size_t)b * P.n_theta + r0) * ndim;
-    for (int i = threadIdx.x; i < kRows * ndim; i += kThreads) prop[i] = (i < n * ndim) ? th[i] : 0.0;
-    __syncthreads();
-    vec_prepare_rows<Row>(s, P.d.n_modes, prop, ndim, n);
-    __syncthreads();
-    if (WANT_Z) {
-      vec_eval_Z<Row>(s, N, P.d.n_modes, n, P.Z + ((size_t)b * P.n_theta + r0) * 2 * N);
-    } else {
-      vec_eval_chi<Row>(s, N, P.d.n_modes, n, chi);
-      __syncthreads();
-      for (int q = threadIdx.x; q < n; q += kThreads)
-        P.lp[(size_t)b * P.n_theta + r0 + q] =
-            in_bounds(prop + q * ndim, bnd, ndim) ? -0.5 * (chi[q] + s.llconst) : neg_inf();
-    }
-    __syncthreads();
-  }
+static int launch_vec(const BatchParams& P, cudaStream_t st, const char* name) {
+  return launch_batch<VecEvaluator<Row>, WANT_Z>(P, 8, batch_smem<VecEvaluator<Row>>(P.d), st, name);
 }
 
 template <bool WANT_Z>
 static int run_batch_vec_t(const BatchParams& P, cudaStream_t st) {
-  const size_t smem = batch_other_bytes(P.d) + vec_smem_doubles(P.d.n_freq, kRows, vec_row_consts(P.d)) * 8;
-  int chunks = ceil_div(P.n_theta, kRows);
-  const int cap = max(1, (148 * 8) / max(1, P.B));   // enough CTAs to fill the chip, no more
-  if (chunks > cap) chunks = cap;
-  const dim3 grid(chunks, P.B);
   switch (P.d.model) {
     case BISIP_MODEL_COLECOLE:
       switch (P.d.n_modes) {
-        case 1: return launch(vec_batch_kernel<ColeColeRowT<1>, WANT_Z>, grid, smem, st, "colecole_batch", &P);
-        case 2: return launch(vec_batch_kernel<ColeColeRowT<2>, WANT_Z>, grid, smem, st, "colecole_batch", &P);
-        case 3: return launch(vec_batch_kernel<ColeColeRowT<3>, WANT_Z>, grid, smem, st, "colecole_batch", &P);
-        case 4: return launch(vec_batch_kernel<ColeColeRowT<4>, WANT_Z>, grid, smem, st, "colecole_batch", &P);
+        case 1: return launch_vec<ColeColeRowT<1>, WANT_Z>(P, st, "colecole_batch");
+        case 2: return launch_vec<ColeColeRowT<2>, WANT_Z>(P, st, "colecole_batch");
+        case 3: return launch_vec<ColeColeRowT<3>, WANT_Z>(P, st, "colecole_batch");
+        case 4: return launch_vec<ColeColeRowT<4>, WANT_Z>(P, st, "colecole_batch");
         default:
-          if (P.d.n_modes <= 8) return launch(vec_batch_kernel<ColeColeRow, WANT_Z>, grid, smem, st, "colecole_batch", &P);
-          return launch(vec_batch_kernel<ColeColeRowBig, WANT_Z>, grid, smem, st, "colecole_batch", &P);
+          if (P.d.n_modes <= 8) return launch_vec<ColeColeRow, WANT_Z>(P, st, "colecole_batch");
+          return launch_vec<ColeColeRowBig, WANT_Z>(P, st, "colecole_batch");
       }
-    case BISIP_MODEL_DIAS: return launch(vec_batch_kernel<DiasRow, WANT_Z>, grid, smem, st, "dias_batch", &P);
-    default: return launch(vec_batch_kernel<ShinRow, WANT_Z>, grid, smem, st, "shin_batch", &P);
+    case BISIP_MODEL_DIAS: return launch_vec<DiasRow, WANT_Z>(P, st, "dias_batch");
+    default: return launch_vec<ShinRow, WANT_Z>(P, st, "shin_batch");
   }
 }
 

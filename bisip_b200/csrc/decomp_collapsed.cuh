@@ -43,6 +43,27 @@ __device__ inline double* decomp_c_carve(DecompCSmem& s, double* base, const Dec
   return base;
 }
 
+// G_ic = sum_k L_ik K_kc * is for one column c: frequency wj, real part of K or the imaginary one (imag), lt = row i
+// of L.  Compensated (Dot2, Ogita-Rump-Oishi) sum: sum + comp = the exact dot product to ~1 ulp.
+__device__ __forceinline__ double dot2_lk(const double* __restrict__ lt, const double* __restrict__ taus, int S, double wj,
+                                          double c_exp, double cs, double sn, bool imag, double is) {
+  double sum = 0.0, comp = 0.0;
+  for (int k = 0; k < S; ++k) {
+    double kre, kim;
+    debye_kernel_term(wj, taus[k], c_exp, cs, sn, kre, kim);
+    const double kv = (imag ? kim : kre) * is;
+    const double l = lt[k];
+    const double p = __dmul_rn(l, kv);
+    const double pe = __fma_rn(l, kv, -p);
+    const double t = __dadd_rn(sum, p);
+    const double bb = __dsub_rn(t, sum);
+    const double se = __dadd_rn(__dsub_rn(sum, __dsub_rn(t, bb)), __dsub_rn(p, bb));
+    sum = t;
+    comp = __dadd_rn(comp, __dadd_rn(se, pe));
+  }
+  return sum + comp;
+}
+
 // Per-spectrum constants.  All threads of the CTA (any CTA size); ends with __syncthreads().
 // Likelihood mode (y != nullptr): G and the data term are pre-scaled by 1/sigma_c exactly as
 // decomp_init() pre-scales K, so the dot product yields the normalised residual directly.
@@ -76,22 +97,7 @@ __device__ inline void decomp_c_init(DecompCSmem& s, const DecompCShape& sh, dou
       const int j = c < N ? c : c - N;
       const double wj = w[j];
       const double is = scaled ? 1.0 / yerr[c] : 1.0;
-      const double* lt = log_taus + (size_t)i * S;
-      double sum = 0.0, comp = 0.0;                  // Dot2 (Ogita-Rump-Oishi): sum + comp = exact dot to ~1 ulp
-      for (int k = 0; k < S; ++k) {
-        double kre, kim;
-        debye_kernel_term(wj, taus[k], c_exp, cs, sn, kre, kim);
-        const double kv = (c < N ? kre : kim) * is;
-        const double l = lt[k];
-        const double p = __dmul_rn(l, kv);
-        const double pe = __fma_rn(l, kv, -p);
-        const double t = __dadd_rn(sum, p);
-        const double bb = __dsub_rn(t, sum);
-        const double se = __dadd_rn(__dsub_rn(sum, __dsub_rn(t, bb)), __dsub_rn(p, bb));
-        sum = t;
-        comp = __dadd_rn(comp, __dadd_rn(se, pe));
-      }
-      g = sum + comp;
+      g = dot2_lk(log_taus + (size_t)i * S, taus, S, wj, c_exp, cs, sn, c >= N, is);
     }
     s.rec[(size_t)c * kCRec + 2 + i] = g;
   }
@@ -241,18 +247,6 @@ __device__ __forceinline__ int decomp_c_ngroups(int rows_cap, int N) {
   DecompCPlan pl;
   pl.make(rows_cap, N);
   return pl.ngroups;
-}
-
-// chi[row] = sum_c ((y_c - Z_c)/sigma_c)^2 (batched log-probability kernel).  chi[] is written but not synchronised.
-__device__ inline void decomp_c_eval_chi(const DecompCSmem& s, const DecompCShape& sh, const double* __restrict__ prop,
-                                         int ndim, int nrows, int rows_pad, double* chi) {
-  const int ngroups = decomp_c_eval_parts(s, sh, rows_pad, prop, ndim, nrows, rows_pad);
-  __syncthreads();
-  for (int p = threadIdx.x; p < nrows; p += blockDim.x) {
-    double acc = 0.0;
-    for (int g = 0; g < ngroups; ++g) acc += s.part[(size_t)g * rows_pad + p];
-    chi[p] = acc;
-  }
 }
 
 // Forward only (decomp_c_init with y == nullptr): Z[row][2][N] = R0*(delta_c - z_c), coalesced over columns.

@@ -195,6 +195,7 @@ __device__ __forceinline__ int decomp_iters_per_warp(const DecompShape& sh, int 
 }
 struct NoSide {
   __device__ __forceinline__ void advance() {}
+  __device__ __forceinline__ void finish() {}
 };
 
 template <int KC, class Side>

@@ -27,6 +27,13 @@ inline int device_smem_optin() {
   return v;
 }
 
+inline int device_sm_count() {
+  int dev = 0, v = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) return 0;
+  cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev);
+  return v;
+}
+
 template <typename K>
 int launch(K kernel, dim3 grid, size_t smem, cudaStream_t st, const char* name, const void* params_ptr,
            int threads = kThreads) {

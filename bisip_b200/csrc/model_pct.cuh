@@ -12,7 +12,7 @@
 //     (decomp_collapsed.cuh) — FP64 for every `precision`, within 1e-12 of the two-stage forward.
 #pragma once
 #include "common.cuh"
-#include "decomp_eval.cuh"
+#include "decomp_collapsed.cuh"
 #include "models.cuh"
 #include "stats.cuh"
 
@@ -75,22 +75,7 @@ __global__ void __launch_bounds__(kStatThreads, 1) model_percentile_kernel(const
     if (tid < D) {
       double cs, sn;
       sincospi(0.5 * P.d.c_exp, &sn, &cs);
-      const double* lt = lts + (size_t)tid * S;
-      double sum = 0.0, comp = 0.0;                    // Dot2, as decomp_c_init
-      for (int k = 0; k < S; ++k) {
-        double kre, kim;
-        debye_kernel_term(wj, taus[k], P.d.c_exp, cs, sn, kre, kim);
-        const double kv = imag ? kim : kre;
-        const double l = lt[k];
-        const double p = __dmul_rn(l, kv);
-        const double pe = __fma_rn(l, kv, -p);
-        const double t = __dadd_rn(sum, p);
-        const double bb = __dsub_rn(t, sum);
-        const double se = __dadd_rn(__dsub_rn(sum, __dsub_rn(t, bb)), __dsub_rn(p, bb));
-        sum = t;
-        comp = __dadd_rn(comp, __dadd_rn(se, pe));
-      }
-      s_g[tid] = sum + comp;
+      s_g[tid] = dot2_lk(lts + (size_t)tid * S, taus, S, wj, P.d.c_exp, cs, sn, imag, 1.0);
     }
   } else if (tid == 0) {
     s_fq[0] = wj; s_fq[1] = sqrt(wj); s_fq[2] = log(wj); s_fq[3] = 0.0;

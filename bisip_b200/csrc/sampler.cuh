@@ -528,8 +528,12 @@ struct DecompEvaluator {
   __device__ double llconst() const { return sm.llconst; }
   __device__ __forceinline__ double chi_of(const double* chi, int q) const { return chi[q]; }
   __device__ int iters_per_warp(int nrows) const { return decomp_iters_per_warp(sh, nrows); }
-  __device__ void eval_chi(const double* prop, int ndim, int nrows, double* chi, RankSide& side) {
+  template <class Side>
+  __device__ void eval_chi(const double* prop, int ndim, int nrows, double* chi, Side& side) {
     decomp_eval_chi<KC>(sm, sh, prop, ndim, nrows, rows_pad, chi, side);
+  }
+  __device__ void eval_Z(const double* prop, int ndim, int nrows, double* Z) {
+    decomp_eval_Z<KC>(sm, sh, prop, ndim, nrows, Z);
   }
 };
 
@@ -556,9 +560,13 @@ struct DecompRCEvaluator {
   __device__ double llconst() const { return sm.llconst; }
   __device__ __forceinline__ double chi_of(const double* chi, int q) const { return chi[q]; }
   __device__ int iters_per_warp(int) const { return 0; }
-  __device__ void eval_chi(const double* prop, int ndim, int nrows, double* chi, RankSide& side) {
+  template <class Side>
+  __device__ void eval_chi(const double* prop, int ndim, int nrows, double* chi, Side& side) {
     side.finish();
     decomp_rc_eval_chi(sm, sh, prop, ndim, nrows, rows_pad, chi);
+  }
+  __device__ void eval_Z(const double* prop, int ndim, int nrows, double* Z) {
+    decomp_rc_eval_Z(sm, sh, prop, ndim, nrows, Z);
   }
 };
 
@@ -586,9 +594,13 @@ struct DecompTF32Evaluator {
   __device__ double llconst() const { return sm.llconst; }
   __device__ __forceinline__ double chi_of(const double* chi, int q) const { return chi[q]; }
   __device__ int iters_per_warp(int) const { return 0; }
-  __device__ void eval_chi(const double* prop, int ndim, int nrows, double* chi, RankSide& side) {
+  template <class Side>
+  __device__ void eval_chi(const double* prop, int ndim, int nrows, double* chi, Side& side) {
     side.finish();
     decomp_tf32_eval_chi<PREC>(sm, sh, prop, ndim, nrows, rows_pad, chi);
+  }
+  __device__ void eval_Z(const double* prop, int ndim, int nrows, double* Z) {
+    decomp_tf32_eval_Z<PREC>(sm, sh, prop, ndim, nrows, Z);
   }
 };
 
@@ -615,9 +627,13 @@ struct DecompUmmaEvaluator {
   __device__ double llconst() const { return sm.llconst; }
   __device__ __forceinline__ double chi_of(const double* chi, int q) const { return chi[q]; }
   __device__ int iters_per_warp(int) const { return 0; }
-  __device__ void eval_chi(const double* prop, int ndim, int nrows, double* chi, RankSide& side) {
+  template <class Side>
+  __device__ void eval_chi(const double* prop, int ndim, int nrows, double* chi, Side& side) {
     side.finish();
     decomp_umma_eval<PREC, false>(sm, sh, prop, ndim, nrows, chi, nullptr);
+  }
+  __device__ void eval_Z(const double* prop, int ndim, int nrows, double* Z) {
+    decomp_umma_eval<PREC, true>(sm, sh, prop, ndim, nrows, nullptr, Z);
   }
   __device__ void release() { decomp_umma_release(sm, sh); }   // frees the tensor memory
 };
@@ -653,9 +669,13 @@ struct DecompCollapsedEvaluator {
     return acc;
   }
   __device__ int iters_per_warp(int) const { return 0; }
-  __device__ void eval_chi(const double* prop, int ndim, int nrows, double* chi, RankSide& side) {
+  template <class Side>
+  __device__ void eval_chi(const double* prop, int ndim, int nrows, double* chi, Side& side) {
     side.finish();
     decomp_c_eval_parts(sm, sh, rows_pad, prop, ndim, nrows, rows_pad);
+  }
+  __device__ void eval_Z(const double* prop, int ndim, int nrows, double* Z) {
+    decomp_c_eval_Z(sm, sh, prop, ndim, nrows, Z);
   }
 };
 
@@ -684,10 +704,12 @@ struct VecEvaluator {
     Row::prepare(th, n_modes, sm.rowc + (size_t)q * Row::kRC);
   }
   __device__ __forceinline__ void release() {}
-  __device__ void eval_chi(const double*, int, int nrows, double* chi, RankSide& side) {
+  template <class Side>
+  __device__ void eval_chi(const double*, int, int nrows, double* chi, Side& side) {
     side.finish();
     vec_eval_chi<Row, ILP>(sm, N, n_modes, nrows, chi);
   }
+  __device__ void eval_Z(const double*, int, int nrows, double* Z) { vec_eval_Z<Row>(sm, N, n_modes, nrows, Z); }
 };
 
 // Co-resident CTAs that start together stay phase-locked: both run their serial phases
