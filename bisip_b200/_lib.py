@@ -24,7 +24,7 @@ EXPORTS = ("bisip_abi_version", "bisip_last_error", "bisip_launch_count", "bisip
            "bisip_log_probability", "bisip_decomp_build_kernel", "bisip_n_keep",
            "bisip_ensemble_run", "bisip_column_stats_workspace", "bisip_column_stats",
            "bisip_decomp_kernel_kind", "bisip_model_percentile", "bisip_gauss_loglike",
-           "bisip_autocorr_time")
+           "bisip_autocorr_time", "bisip_rtd_stats")
 KERNEL_KINDS = {0: "dmma", 1: "dmma-cluster", 2: "mma-tf32", 3: "tcgen05", 4: "tcgen05-cluster", 5: "fp64-collapsed"}
 
 
@@ -82,6 +82,9 @@ def load():
                                            C.POINTER(C.c_int64), C.POINTER(C.c_double), vp, vp]
     lib.bisip_autocorr_time.restype = C.c_int
     lib.bisip_autocorr_time.argtypes = [vp, i32, i32, i32, i32, dbl, vp, vp]
+    lib.bisip_rtd_stats.restype = C.c_int
+    lib.bisip_rtd_stats.argtypes = [i32, i64, i32, i32, i32, vp, vp, i64, i32, C.POINTER(C.c_int64),
+                                    C.POINTER(C.c_double), vp, vp, vp, vp]
     if lib.bisip_abi_version() != ABI_VERSION:
         raise BisipError("libbisip_b200.so ABI version mismatch")
     _lib = lib

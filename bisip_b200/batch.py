@@ -15,6 +15,7 @@ the *global* spectrum index, so results do not depend on ``G`` or on the sub-bat
 the kept chains).  ``gather`` is the per-tensor variant (NCCL on GPU tensors; gloo on CPU tensors in the unit tests).
 """
 import os
+from dataclasses import replace
 
 import numpy as np
 import torch
@@ -132,7 +133,7 @@ def gather_chain_to_rank0(chain, n_total, rank, world, group=None, chunk_bytes=1
 
 
 def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 97.5), p0=None, gather_chain=False,
-                group=None, batch_size=None, autocorr=False, **kwargs):
+                group=None, batch_size=None, autocorr=False, rtd=False, model_curves=False, **kwargs):
     """Invert a whole survey on all ranks of the current ``torch.distributed`` job (one process per GPU).
 
     The reference inverts a batch as a serial loop over files (``docs/tutorials/decomposition.ipynb`` cells 9-10);
@@ -140,8 +141,9 @@ def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 9
     (B, W, ndim)), inverts its contiguous block ``shard_range(B, rank, world)`` with ``BatchInversion`` (Philox
     counters carry the global spectrum index: the result does not depend on the number of ranks), and the
     per-spectrum summaries are all-gathered with one NCCL collective, so every rank returns the complete result:
-    ``percentiles`` (B, len(p), ndim), ``mean``, ``std`` (B, ndim), ``acceptance_fraction``, ``flags`` (B,), and with
-    ``autocorr=True`` ``autocorr_time`` (B, ndim) (see ``BatchInversion.fit``).  With ``gather_chain=True`` the kept
+    ``percentiles`` (B, len(p), ndim), ``mean``, ``std`` (B, ndim), ``acceptance_fraction``, ``flags`` (B,), with
+    ``autocorr=True`` ``autocorr_time`` (B, ndim), and with ``rtd=True`` / ``model_curves=True`` the RTD,
+    total-chargeability and model-curve keys (see ``BatchInversion.fit``).  With ``gather_chain=True`` the kept
     chains (``discard`` / ``thin``) are gathered to rank 0 in chunks (``chain`` (B, n_keep, W, ndim) on rank 0, None
     elsewhere).  Without an initialised process group it runs the
     whole survey on the current device.  ``kwargs`` go to ``BatchInversion`` (nwalkers, nsteps, poly_deg, ...)."""
@@ -154,9 +156,10 @@ def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 9
     w_arr = np.asarray(w, dtype=np.float64)
     inv = BatchInversion(model, w_arr if w_arr.ndim == 1 else w_arr[lo:hi], zn[lo:hi], zn_err[lo:hi],
                          spectrum_offset=lo + int(kwargs.pop('spectrum_offset', 0)), **kwargs)
-    # autocorr is passed only when set, so fit_device overrides written for the older signature keep working
+    # the optional products are passed only when set, so fit_device overrides written for the older signature keep working
+    extra = {k: True for k, on in (('autocorr', autocorr), ('rtd', rtd), ('model_curves', model_curves)) if on}
     dev_res = inv.fit_device(None if p0 is None else p0[lo:hi], discard, thin, percentiles, gather_chain, batch_size,
-                             **({'autocorr': True} if autocorr else {}))
+                             **extra)
     chain = dev_res.pop('chain', None)
     dev_res.pop('log_prob', None)
     if on and world > 1:
@@ -284,7 +287,7 @@ class BatchInversion:
 
     # ------------------------------------------------------------------ fit
     def fit(self, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), keep_chain=False, batch_size=None,
-            autocorr=False):
+            autocorr=False, rtd=False, model_curves=False):
         """Sample every spectrum and summarise the kept chain on the device.
 
         Returns (and stores in ``self.results``) a dict of host arrays:
@@ -294,9 +297,17 @@ class BatchInversion:
         With ``autocorr=True`` also ``autocorr_time`` (B, ndim): emcee's integrated autocorrelation time of every
         parameter in steps (``sampler.get_autocorr_time(discard=, thin=, quiet=True)`` of each spectrum), computed on
         the device from each sub-batch's kept chain before it is dropped; NaN where a walker's kept series is constant.
+        With ``rtd=True`` (``'decomp'`` only) the relaxation-time distribution m_l = sum_i a_i log_tau_l^i and the total
+        chargeability sum_l m_l of every kept sample are summarised like the parameters: ``rtd_percentiles``
+        (B, len(p), n_tau), ``rtd_mean``, ``rtd_std`` (B, n_tau), ``total_chargeability_percentiles`` (B, len(p)),
+        ``total_chargeability_mean``, ``total_chargeability_std`` (B,).  The RTD percentiles equal ``np.percentile`` of
+        ``products.relaxation_time_distribution`` over the flat chain bit for bit.
+        With ``model_curves=True`` also ``model_percentiles`` (B, len(p), 2, N): the percentiles of the forward model
+        over the flat chain in normalised units, as ``get_model_percentile`` (FP64 for every ``precision``).
+        Both are computed on the device from each sub-batch's kept chain before it is dropped.
         """
         dev_res = self.fit_device(p0, discard, thin, percentiles, keep_chain, batch_size, _chain_to_host=True,
-                                  autocorr=autocorr)
+                                  autocorr=autocorr, rtd=rtd, model_curves=model_curves)
         self.percentiles = tuple(float(q) for q in percentiles)
         self.results = {k: (v if isinstance(v, np.ndarray) else v.cpu().numpy()) for k, v in dev_res.items()}
         self._apply_nan_policy(self.results['flags'])
@@ -313,13 +324,14 @@ class BatchInversion:
             warnings.warn(msg, RuntimeWarning)
 
     def fit_gathered(self, n_total, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), group=None, batch_size=None,
-                     autocorr=False):
+                     autocorr=False, rtd=False, model_curves=False):
         """``fit`` for a shard-local inversion inside a ``torch.distributed`` job: this object holds spectra
         ``[spectrum_offset, spectrum_offset + n_spectra)`` of a survey of ``n_total`` sharded by ``shard_range``; after
         sampling, the summaries of all ranks are all-gathered (one NCCL collective) and the COMPLETE result
         (``n_total`` rows, host arrays) is returned on every rank.  Without a process group it equals ``fit``."""
         import torch.distributed as dist
-        dev_res = self.fit_device(p0, discard, thin, percentiles, False, batch_size, autocorr=autocorr)
+        dev_res = self.fit_device(p0, discard, thin, percentiles, False, batch_size, autocorr=autocorr, rtd=rtd,
+                                  model_curves=model_curves)
         if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
             dev_res = gather_packed(dev_res, int(n_total), dist.get_rank(group), dist.get_world_size(group), group)
         self.percentiles = tuple(float(q) for q in percentiles)
@@ -328,9 +340,11 @@ class BatchInversion:
         return self.results
 
     def fit_device(self, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), keep_chain=False,
-                   batch_size=None, _chain_to_host=False, autocorr=False):
+                   batch_size=None, _chain_to_host=False, autocorr=False, rtd=False, model_curves=False):
         """Same as ``fit`` but leaves the summaries on the GPU (for the NCCL gather).  With ``keep_chain`` the kept
         chains of all sub-batches stay on the device too (``fit`` moves each sub-batch's chain to the host instead)."""
+        if rtd and self.model != 'decomp':
+            raise ValueError("rtd=True is defined for the polynomial decomposition ('decomp') only")
         B, W, ndim = self.n_spectra, self.nwalkers, self.ndim
         nk = engine.n_keep(self.nsteps, discard, thin)
         if nk == 0:
@@ -343,6 +357,15 @@ class BatchInversion:
                    'flags': torch.empty((0,), dtype=torch.int32, device=self.device)}
             if autocorr:
                 out['autocorr_time'] = torch.empty((0, ndim), **f64)
+            P = len(percentiles)
+            if rtd:
+                S = self.log_taus.shape[-1]
+                out.update(rtd_percentiles=torch.empty((0, P, S), **f64), rtd_mean=torch.empty((0, S), **f64),
+                           rtd_std=torch.empty((0, S), **f64), total_chargeability_percentiles=torch.empty((0, P), **f64),
+                           total_chargeability_mean=torch.empty((0,), **f64),
+                           total_chargeability_std=torch.empty((0,), **f64))
+            if model_curves:
+                out['model_percentiles'] = torch.empty((0, P, 2, self.w.shape[-1]), **f64)
             if keep_chain:
                 out['chain'], out['log_prob'] = torch.empty((0, nk, W, ndim), **f64), torch.empty((0, nk, W), **f64)
                 if _chain_to_host:
@@ -355,6 +378,12 @@ class BatchInversion:
         acc = {k: [] for k in ('percentiles', 'mean', 'std', 'acceptance_fraction', 'flags')}
         if autocorr:
             acc['autocorr_time'] = []
+        if rtd:
+            for k in ('rtd_percentiles', 'rtd_mean', 'rtd_std', 'total_chargeability_percentiles',
+                      'total_chargeability_mean', 'total_chargeability_std'):
+                acc[k] = []
+        if model_curves:
+            acc['model_percentiles'] = []
         if keep_chain:
             acc['chain'], acc['log_prob'] = [], []
         for lo in range(0, B, bs):
@@ -370,16 +399,28 @@ class BatchInversion:
                     raise ValueError("At least one parameter value was infinite or NaN")
             else:
                 coords = _lib.dev_f64(self.draw_p0(lo, hi), self.device)
-            res = engine.ensemble_run(self._spec(lo, hi), coords, w, y, ye, bounds, nsteps=self.nsteps, seed=self.seed,
+            spec = self._spec(lo, hi)
+            res = engine.ensemble_run(spec, coords, w, y, ye, bounds, nsteps=self.nsteps, seed=self.seed,
                                       spectrum0=self.spectrum_offset + lo, a=self.a, discard=discard, thin=thin,
                                       store_chain=True, store_logp=keep_chain)
-            st = engine.column_stats(res['chain'].reshape(hi - lo, nk * W, ndim), p=list(percentiles),
-                                     want_mean=True, want_std=True)
+            flat = res['chain'].reshape(hi - lo, nk * W, ndim)
+            st = engine.column_stats(flat, p=list(percentiles), want_mean=True, want_std=True)
             acc['percentiles'].append(st['pct'])
             acc['mean'].append(st['mean'])
             acc['std'].append(st['std'])
             if autocorr:                           # emcee's default c = 5; in steps of the run
                 acc['autocorr_time'].append(thin * engine.autocorr_time(res['chain'], 5.0))
+            if rtd:                                # column n_tau of rtd_stats is the total chargeability
+                S = spec.log_taus.shape[-1]
+                rs = engine.rtd_stats(flat, spec.log_taus, p=list(percentiles), want_mean=True, want_std=True)
+                acc['rtd_percentiles'].append(rs['pct'][:, :, :S])
+                acc['rtd_mean'].append(rs['mean'][:, :S])
+                acc['rtd_std'].append(rs['std'][:, :S])
+                acc['total_chargeability_percentiles'].append(rs['pct'][:, :, S])
+                acc['total_chargeability_mean'].append(rs['mean'][:, S])
+                acc['total_chargeability_std'].append(rs['std'][:, S])
+            if model_curves:
+                acc['model_percentiles'].append(self._model_curves(spec, flat, w, percentiles))
             acc['acceptance_fraction'].append(res['accepted'].to(torch.float64).mean(1) / float(self.nsteps))
             acc['flags'].append(res['flags'])
             if keep_chain and _chain_to_host:      # sub-batching stays effective: nothing accumulates on the device
@@ -389,6 +430,29 @@ class BatchInversion:
                 acc['chain'].append(res['chain'])
                 acc['log_prob'].append(res['log_prob'])
         return {k: (np.concatenate(v, 0) if isinstance(v[0], np.ndarray) else torch.cat(v, 0)) for k, v in acc.items()}
+
+    MODEL_CURVE_BYTES = 1 << 30    # (n, 2N) model matrices of one group of the model-curve fallback
+
+    def _model_curves(self, spec, flat, w, percentiles):
+        """Percentiles of the forward model over every spectrum's flat chain, (k, len(p), 2, N): fused
+        (``engine.model_percentile``), or for chains past one CTA's shared memory ``forward`` + ``column_stats`` on
+        groups of spectra whose model matrices fit ``MODEL_CURVE_BYTES``.  FP64 on both paths, as the fused kernel."""
+        p = list(percentiles)
+        out = engine.model_percentile(spec, flat, w, p)
+        if out is not None:
+            return out
+        if spec.precision not in (_lib.PREC_FP64, _lib.PREC_FP64_COLLAPSED):
+            spec = replace(spec, precision=_lib.PREC_FP64)
+        k, n, _ = flat.shape
+        N = w.shape[-1]
+        g = max(1, self.MODEL_CURVE_BYTES // (n * 2 * N * 8))
+        parts = []
+        for s0 in range(0, k, g):
+            s1 = min(k, s0 + g)
+            sub = spec if spec.tau_stride() == 0 else replace(spec, taus=spec.taus[s0:s1], log_taus=spec.log_taus[s0:s1])
+            Z = engine.forward(sub, flat[s0:s1], w if w.dim() == 1 else w[s0:s1])
+            parts.append(engine.column_stats(Z.reshape(s1 - s0, n, 2 * N), p=p)['pct'].reshape(s1 - s0, -1, 2, N))
+        return torch.cat(parts, 0)
 
     # ------------------------------------------------------------------ results
     def rtd(self, stat='mean'):

@@ -10,6 +10,7 @@
 #include "stats.cuh"
 #include "model_pct.cuh"
 #include "autocorr.cuh"
+#include "rtd_stats.cuh"
 
 namespace bisip {
 
@@ -367,6 +368,34 @@ int bisip_autocorr_time(const double* data, int n_spectra, int n_keep, int n_wal
   if (gsmem + kAcfStaticSmem > (size_t)optin)
     return fail(BISIP_ERR_UNSUPPORTED, "bisip_autocorr_time: too many walkers for one CTA's shared memory");
   return launch(autocorr_kernel<false>, grid, gsmem, (cudaStream_t)stream, "autocorr_time", &P, kAcfThreads);
+}
+
+int bisip_rtd_stats(int n_spectra, int64_t n_samples, int ndim, int n_coef, int n_tau, const double* theta,
+                    const double* log_taus, int64_t tau_stride, int n_pct, const int64_t* pct_lo, const double* pct_gamma,
+                    double* pct_out, double* mean_out, double* std_out, void* stream) {
+  if (!theta || !log_taus || n_spectra <= 0 || n_samples <= 0 || ndim <= 0 || n_coef <= 0 || n_tau <= 0 ||
+      tau_stride < 0 || n_pct < 0)
+    return fail(BISIP_ERR_BAD_ARG, "bisip_rtd_stats: bad argument");
+  if (n_coef > kMaxCoefPct) return fail(BISIP_ERR_UNSUPPORTED, "bisip_rtd_stats: n_coef > 32");
+  if (ndim != 1 + n_coef) return fail(BISIP_ERR_BAD_ARG, "bisip_rtd_stats: ndim != 1 + n_coef");
+  if (n_pct > 0 && (!pct_lo || !pct_gamma || !pct_out))
+    return fail(BISIP_ERR_BAD_ARG, "bisip_rtd_stats: percentile arrays null");
+  if (n_pct == 0 && !mean_out && !std_out) return fail(BISIP_ERR_BAD_ARG, "bisip_rtd_stats: no output requested");
+  if (n_pct > kMaxPct) return fail(BISIP_ERR_UNSUPPORTED, "bisip_rtd_stats: at most 16 percentiles per call");
+  if (n_spectra > 65535) return fail(BISIP_ERR_UNSUPPORTED, "bisip_rtd_stats: n_spectra > 65535 per call");
+  if (n_tau > 0x7ffffffe) return fail(BISIP_ERR_UNSUPPORTED, "bisip_rtd_stats: n_tau + 1 columns exceed the grid");
+  DeviceGuard guard(theta);
+  RtdParams P;
+  P.theta = theta; P.log_taus = log_taus; P.tau_stride = tau_stride;
+  P.ndim = ndim; P.n_coef = n_coef; P.n_tau = n_tau;
+  P.st.data = nullptr; P.st.n = n_samples; P.st.ncol = n_tau + 1; P.st.B = n_spectra; P.st.npct = n_pct;
+  for (int i = 0; i < n_pct; ++i) { P.st.lo[i] = pct_lo[i]; P.st.gamma[i] = pct_gamma[i]; }
+  P.st.pct_out = n_pct ? pct_out : nullptr; P.st.mean_out = mean_out; P.st.std_out = std_out;
+  const dim3 grid(n_tau + 1, n_spectra);
+  size_t smem = 0;
+  if (stats_fits_smem(n_samples, 2 * n_pct, &smem))
+    return launch(rtd_stats_smem_kernel, grid, smem, (cudaStream_t)stream, "rtd_stats", &P, kStatThreads);
+  return launch(rtd_stats_global_kernel, grid, 0, (cudaStream_t)stream, "rtd_stats", &P, kThreads);
 }
 
 }  // extern "C"

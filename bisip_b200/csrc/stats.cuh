@@ -338,19 +338,15 @@ __global__ void __launch_bounds__(kStatThreads, 1) column_stats_smem_kernel(cons
                         P.ncol, P.mean_out ? P.mean_out + o : nullptr, P.std_out ? P.std_out + o : nullptr, hist, pool, red);
 }
 
-// Columns that do not fit in shared memory: the same statistics straight from global memory (strided reads, the
-// generic radix select).  grid (ncol, B), kThreads threads.
-__global__ void __launch_bounds__(kThreads) column_stats_global_kernel(const StatsParams P) {
-  __shared__ unsigned int hist[kMaxRanks * 256];
+// Statistics of a column of any length read through load(i), i in [0, n): the two-pass mean / std and the generic
+// radix select, without a copy of the column.  pct_out[q * pct_stride]; all threads; needs `red` [32] and `hist`
+// [kMaxRanks * 256].
+template <int NT, class Load>
+__device__ void global_column_stats(Load load, long long n, const StatsParams& P, double* pct_out, long long pct_stride,
+                                    double* mean_out, double* std_out, unsigned int* hist, double* red) {
   __shared__ long long s_krank[kMaxRanks];
   __shared__ double s_ans[kMaxRanks];
-  __shared__ double red[32];
-  constexpr int NT = kThreads;
-  const int col = blockIdx.x, b = blockIdx.y, tid = threadIdx.x;
-  const long long n = P.n;
-  const double* src = P.data + (size_t)b * n * P.ncol + col;
-  const size_t stride = P.ncol;
-  auto load = [&](long long i) { return __ldg(src + (size_t)i * stride); };
+  const int tid = threadIdx.x;
   double s = 0.0;
   int nan = 0;
   for (long long i = tid; i < n; i += NT) {
@@ -360,7 +356,7 @@ __global__ void __launch_bounds__(kThreads) column_stats_global_kernel(const Sta
   }
   const double mean = block_sum_nt<NT>(s, red) / (double)n;
   const bool has_nan = __syncthreads_or(nan) != 0;
-  if (P.mean_out != nullptr || P.std_out != nullptr) {
+  if (mean_out != nullptr || std_out != nullptr) {
     double v = 0.0;
     for (long long i = tid; i < n; i += NT) {
       const double d = load(i) - mean;
@@ -368,8 +364,8 @@ __global__ void __launch_bounds__(kThreads) column_stats_global_kernel(const Sta
     }
     const double var = block_sum_nt<NT>(v, red) / (double)n;
     if (tid == 0) {
-      if (P.mean_out) P.mean_out[(size_t)b * P.ncol + col] = mean;
-      if (P.std_out) P.std_out[(size_t)b * P.ncol + col] = sqrt(var);
+      if (mean_out) *mean_out = mean;
+      if (std_out) *std_out = sqrt(var);
     }
   }
   const int R = 2 * P.npct;
@@ -381,13 +377,26 @@ __global__ void __launch_bounds__(kThreads) column_stats_global_kernel(const Sta
     s_krank[tid] = k;
   }
   __syncthreads();
-  double* out = P.pct_out + (size_t)b * P.npct * P.ncol + col;
   if (has_nan) {
-    if (tid < P.npct) out[(size_t)tid * P.ncol] = __longlong_as_double(0x7ff8000000000000LL);
+    if (tid < P.npct) pct_out[(size_t)tid * pct_stride] = __longlong_as_double(0x7ff8000000000000LL);
     return;
   }
   radix_select_ranks<NT>(load, n, R, s_krank, s_ans, hist);
-  if (tid < P.npct) out[(size_t)tid * P.ncol] = numpy_lerp(s_ans[2 * tid], s_ans[2 * tid + 1], P.gamma[tid]);
+  if (tid < P.npct) pct_out[(size_t)tid * pct_stride] = numpy_lerp(s_ans[2 * tid], s_ans[2 * tid + 1], P.gamma[tid]);
+}
+
+// Columns that do not fit in shared memory: the same statistics straight from global memory (strided reads, the
+// generic radix select).  grid (ncol, B), kThreads threads.
+__global__ void __launch_bounds__(kThreads) column_stats_global_kernel(const StatsParams P) {
+  __shared__ unsigned int hist[kMaxRanks * 256];
+  __shared__ double red[32];
+  const int col = blockIdx.x, b = blockIdx.y;
+  const double* src = P.data + (size_t)b * P.n * P.ncol + col;
+  const size_t stride = P.ncol;
+  auto load = [&](long long i) { return __ldg(src + (size_t)i * stride); };
+  const size_t o = (size_t)b * P.ncol + col;
+  global_column_stats<kThreads>(load, P.n, P, P.pct_out ? P.pct_out + (size_t)b * P.npct * P.ncol + col : nullptr, P.ncol,
+                                P.mean_out ? P.mean_out + o : nullptr, P.std_out ? P.std_out + o : nullptr, hist, red);
 }
 
 }  // namespace bisip

@@ -207,6 +207,51 @@ def autocorr_time(chain, c=5.0):
     return out
 
 
+def rtd_stats(theta, log_taus, p=None, want_mean=False, want_std=False):
+    """Relaxation-time distribution and total chargeability of a decomposition over parameter vectors
+    (``bisip_rtd_stats``; ``theta`` is read in place): theta (B, n, 1 + n_coef), log_taus (n_coef, n_tau) or
+    (B, n_coef, n_tau) -> dict(pct (B, len(p), n_tau + 1), mean (B, n_tau + 1), std (B, n_tau + 1)).  Columns
+    [0, n_tau) are the RTD m_l = sum_i a_i log_taus[i, l], equal to ``products.relaxation_time_distribution`` bit for
+    bit; column n_tau is the total chargeability sum_l m_l.  Statistics over axis 1 as ``column_stats``."""
+    lib = _lib.load()
+    _chk_cuda_f64(theta, log_taus)
+    B, n, ndim = theta.shape
+    n_coef, n_tau = int(log_taus.shape[-2]), int(log_taus.shape[-1])
+    if ndim != 1 + n_coef:
+        raise ValueError(f"expected {n_coef} coefficients, got {ndim - 1}")
+    tau_stride = 0 if log_taus.dim() == 2 else n_tau
+    dev = theta.device
+    p_arr = np.atleast_1d(np.asarray(p, dtype=np.float64)) if p is not None else np.empty(0)
+    npct = int(p_arr.shape[0])
+    C_out = n_tau + 1
+    pct = torch.empty((B, npct, C_out), dtype=torch.float64, device=dev) if npct else None
+    mean = torch.empty((B, C_out), dtype=torch.float64, device=dev) if want_mean else None
+    std = torch.empty((B, C_out), dtype=torch.float64, device=dev) if want_std else None
+    chunks = [(q0, p_arr[q0:q0 + _lib.MAX_PCT]) for q0 in range(0, npct, _lib.MAX_PCT)] or [(0, p_arr)]
+    for s0 in range(0, B, 65535):                  # one launch per 65,535 spectra (grid y) and 16 percentiles
+        k = min(65535, B - s0)
+        lt = log_taus if tau_stride == 0 else log_taus[s0:s0 + k]
+        for i, (q0, pp) in enumerate(chunks):
+            m = int(pp.shape[0])
+            if m:
+                lo, gamma = _lib.percentile_indices(n, pp)
+                lo_c = (C.c_int64 * m)(*[int(v) for v in lo])
+                ga_c = (C.c_double * m)(*[float(v) for v in gamma])
+                whole = m == npct and k == B           # the usual case: the kernel writes straight into the result
+                part = pct if whole else torch.empty((k, m, C_out), dtype=torch.float64, device=dev)
+            else:
+                lo_c = ga_c = part = None
+            first = i == 0                         # mean / std with the first percentile block only
+            rc = lib.bisip_rtd_stats(k, n, ndim, n_coef, n_tau, _lib.ptr(theta[s0:s0 + k]), _lib.ptr(lt), tau_stride,
+                                     m, lo_c, ga_c, _lib.ptr(part),
+                                     _lib.ptr(mean[s0:s0 + k] if first and want_mean else None),
+                                     _lib.ptr(std[s0:s0 + k] if first and want_std else None), _lib.stream_ptr(dev))
+            _lib.check(rc, "bisip_rtd_stats")
+            if m and not whole:
+                pct[s0:s0 + k, q0:q0 + m] = part
+    return {"pct": pct, "mean": mean, "std": std}
+
+
 def model_percentile(spec, theta, w, p):
     """Percentiles of the forward model over parameter vectors, fused (``bisip_model_percentile``): theta (B, n, ndim),
     w (N,) or (B, N), p percentiles -> (B, len(p), 2, N).  The (n, 2N) model matrix is never materialised.  Returns None

@@ -258,15 +258,16 @@ class PolynomialDecomposition(Inversion):
 
         With ``p=None`` the RTD of the posterior-mean coefficients, shape ``(n_tau,)`` (the
         tutorial's ``get_m``); with percentiles ``p`` the per-tau percentiles of the RTD over
-        the chain, shape ``(len(p), n_tau)`` (reduced on the GPU by ``bisip_column_stats``).
+        the chain, shape ``(len(p), n_tau)`` (``bisip_rtd_stats`` on the uploaded chain, the kernel behind
+        ``BatchInversion.fit(..., rtd=True)``; equal to ``np.percentile`` of the RTD of every sample bit for bit).
         ``chain`` / ``discard`` / ``thin`` as in ``get_param_mean``."""
         from .products import relaxation_time_distribution
         if p is None:
             return relaxation_time_distribution(self.get_param_mean(chain=chain, **kwargs)[1:], self.log_taus)
         chain = self.parse_chain(chain, **kwargs)
-        m = relaxation_time_distribution(chain[:, 1:], self.log_taus)              # (n, n_tau)
         dev = _lib.require_cuda(getattr(self, "device", None))
-        out = engine.column_stats(_lib.dev_f64(m, dev).reshape(1, m.shape[0], m.shape[1]), p=p)["pct"][0]
+        th = _lib.dev_f64(chain, dev).reshape(1, -1, chain.shape[-1])
+        out = engine.rtd_stats(th, _lib.dev_const(self.log_taus, dev), p=p)["pct"][0, :, :-1]    # the last column: total
         res = out.cpu().numpy()
         return res if np.ndim(p) else res[0]
 

@@ -51,7 +51,9 @@ def load_percentiles_csv(path):
 def batch_table(param_names, results, ids=None, percentiles=(2.5, 50, 97.5)):
     """Flatten ``BatchInversion.results`` into (column names, 2-D array): one row per spectrum with
     id, acceptance fraction, flags, then mean / std / each percentile of every parameter, and — when the results hold
-    ``autocorr_time`` (``fit(..., autocorr=True)``) — one ``<name>_tau`` column per parameter."""
+    ``autocorr_time`` (``fit(..., autocorr=True)``) — one ``<name>_tau`` column per parameter, then — when they hold the
+    total chargeability (``fit(..., rtd=True)``) — ``total_m_mean``, ``total_m_std`` and one ``total_m_p<q>`` per
+    percentile.  The RTD and model-curve arrays stay in ``results``."""
     B = results['mean'].shape[0]
     ids = np.arange(B) if ids is None else np.asarray(ids)
     cols = ['spectrum', 'acceptance_fraction', 'flags']
@@ -66,4 +68,8 @@ def batch_table(param_names, results, ids=None, percentiles=(2.5, 50, 97.5)):
     if 'autocorr_time' in results:
         cols += [f'{n}_tau' for n in param_names]
         blocks.append(results['autocorr_time'])
+    if 'total_chargeability_mean' in results:
+        cols += ['total_m_mean', 'total_m_std'] + [f'total_m_p{q:g}' for q in percentiles]
+        blocks += [results['total_chargeability_mean'][:, None], results['total_chargeability_std'][:, None],
+                   results['total_chargeability_percentiles']]
     return cols, np.concatenate(blocks, axis=1)

@@ -23,6 +23,8 @@
  *   bisip_model_percentile   <- utils.get_model_percentile (utils.py:17-35)
  *   bisip_autocorr_time      <- emcee autocorr.integrated_time, reached through
  *                               sampler.get_autocorr_time (models.py:154-159)
+ *   bisip_rtd_stats          <- relaxation_time_distribution / total_m of decomposition.ipynb
+ *                               cells 25-29 over the chain, then np.percentile / mean / std
  *
  * Layouts (all row-major, float64):
  *   theta   [n_spectra][n_theta][ndim]      parameter vectors (order as the reference's
@@ -211,6 +213,28 @@ int bisip_model_percentile(const bisip_model_desc *desc, int n_spectra, int64_t 
  */
 int bisip_autocorr_time(const double *data, int n_spectra, int n_keep, int n_walkers, int n_cols,
                         double c, double *tau_out, void *stream);
+
+/*
+ * Relaxation-time distribution and total chargeability of a polynomial decomposition over a chain, read in place
+ * (replaces products.relaxation_time_distribution of every flat-chain sample + np.percentile / np.mean / np.std;
+ * reference docs/tutorials/decomposition.ipynb cells 25-29).
+ *   theta    [n_spectra][n_samples][ndim]   r0, a_0 .. a_{n_coef-1} (r0 is not used); ndim == 1 + n_coef
+ *   log_taus [n_coef][n_tau] (tau_stride 0: shared) or per spectrum at b*tau_stride*n_coef, as in bisip_forward
+ * Column l < n_tau: m_l = sum_i a_i log_taus[i][l], accumulated in ascending i from 0 with unfused multiply and add
+ * (products.relaxation_time_distribution's arithmetic: every value equals NumPy's bit for bit).  Column n_tau: the
+ * total chargeability sum_l m_l of the same sample, evaluated as sum_i a_i (sum_l log_taus[i][l]) (equal up to
+ * rounding).  Statistics per column as bisip_column_stats: exact 'linear' percentiles (pct_lo / pct_gamma as there),
+ * mean and population std; a NaN sample gives NaN percentiles.
+ *   pct_out [n_spectra][n_pct][n_tau+1]; mean_out, std_out [n_spectra][n_tau+1] (each may be NULL, not all three)
+ * One launch; columns longer than one CTA's shared memory (~27,000 samples) are read from global memory, with no
+ * workspace and no length limit.
+ * BISIP_ERR_BAD_ARG: null pointer, non-positive size, ndim != 1 + n_coef, tau_stride < 0, no output;
+ * BISIP_ERR_UNSUPPORTED: n_pct > 16, n_spectra > 65535, n_coef > 32.
+ */
+int bisip_rtd_stats(int n_spectra, int64_t n_samples, int ndim, int n_coef, int n_tau,
+                    const double *theta, const double *log_taus, int64_t tau_stride,
+                    int n_pct, const int64_t *pct_lo, const double *pct_gamma,
+                    double *pct_out, double *mean_out, double *std_out, void *stream);
 
 #ifdef __cplusplus
 }
