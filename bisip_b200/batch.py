@@ -133,7 +133,7 @@ def gather_chain_to_rank0(chain, n_total, rank, world, group=None, chunk_bytes=1
 
 
 def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 97.5), p0=None, gather_chain=False,
-                group=None, batch_size=None, autocorr=False, rtd=False, model_curves=False, **kwargs):
+                group=None, batch_size=None, autocorr=False, rtd=False, model_curves=False, waic=False, **kwargs):
     """Invert a whole survey on all ranks of the current ``torch.distributed`` job (one process per GPU).
 
     The reference inverts a batch as a serial loop over files (``docs/tutorials/decomposition.ipynb`` cells 9-10);
@@ -142,8 +142,8 @@ def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 9
     counters carry the global spectrum index: the result does not depend on the number of ranks), and the
     per-spectrum summaries are all-gathered with one NCCL collective, so every rank returns the complete result:
     ``percentiles`` (B, len(p), ndim), ``mean``, ``std`` (B, ndim), ``acceptance_fraction``, ``flags`` (B,), with
-    ``autocorr=True`` ``autocorr_time`` (B, ndim), and with ``rtd=True`` / ``model_curves=True`` the RTD,
-    total-chargeability and model-curve keys (see ``BatchInversion.fit``).  With ``gather_chain=True`` the kept
+    ``autocorr=True`` ``autocorr_time`` (B, ndim), with ``rtd=True`` / ``model_curves=True`` the RTD,
+    total-chargeability and model-curve keys, and with ``waic=True`` the WAIC keys (see ``BatchInversion.fit``).  With ``gather_chain=True`` the kept
     chains (``discard`` / ``thin``) are gathered to rank 0 in chunks (``chain`` (B, n_keep, W, ndim) on rank 0, None
     elsewhere).  Without an initialised process group it runs the
     whole survey on the current device.  ``kwargs`` go to ``BatchInversion`` (nwalkers, nsteps, poly_deg, ...)."""
@@ -157,7 +157,8 @@ def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 9
     inv = BatchInversion(model, w_arr if w_arr.ndim == 1 else w_arr[lo:hi], zn[lo:hi], zn_err[lo:hi],
                          spectrum_offset=lo + int(kwargs.pop('spectrum_offset', 0)), **kwargs)
     # the optional products are passed only when set, so fit_device overrides written for the older signature keep working
-    extra = {k: True for k, on in (('autocorr', autocorr), ('rtd', rtd), ('model_curves', model_curves)) if on}
+    extra = {k: True for k, on in (('autocorr', autocorr), ('rtd', rtd), ('model_curves', model_curves), ('waic', waic))
+             if on}
     dev_res = inv.fit_device(None if p0 is None else p0[lo:hi], discard, thin, percentiles, gather_chain, batch_size,
                              **extra)
     chain = dev_res.pop('chain', None)
@@ -287,7 +288,7 @@ class BatchInversion:
 
     # ------------------------------------------------------------------ fit
     def fit(self, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), keep_chain=False, batch_size=None,
-            autocorr=False, rtd=False, model_curves=False):
+            autocorr=False, rtd=False, model_curves=False, waic=False):
         """Sample every spectrum and summarise the kept chain on the device.
 
         Returns (and stores in ``self.results``) a dict of host arrays:
@@ -305,9 +306,14 @@ class BatchInversion:
         With ``model_curves=True`` also ``model_percentiles`` (B, len(p), 2, N): the percentiles of the forward model
         over the flat chain in normalised units, as ``get_model_percentile`` (FP64 for every ``precision``).
         Both are computed on the device from each sub-batch's kept chain before it is dropped.
+        With ``waic=True`` also the WAIC of every spectrum over its flat chain (``engine.waic``; Watanabe's widely
+        applicable information criterion, as in Vehtari, Gelman & Gabry 2017), for comparing models fitted to the same
+        data (``products.compare_waic``): ``elpd_waic``, ``p_waic``, ``se_elpd_waic`` (B,), ``waic_pointwise`` (B, N)
+        = lppd - p per frequency, and ``waic_n_high_p`` (B,) int32, the number of frequencies with p > 0.4 (where WAIC
+        is unreliable).  FP64 for every ``precision``; one launch per sub-batch.
         """
         dev_res = self.fit_device(p0, discard, thin, percentiles, keep_chain, batch_size, _chain_to_host=True,
-                                  autocorr=autocorr, rtd=rtd, model_curves=model_curves)
+                                  autocorr=autocorr, rtd=rtd, model_curves=model_curves, waic=waic)
         self.percentiles = tuple(float(q) for q in percentiles)
         self.results = {k: (v if isinstance(v, np.ndarray) else v.cpu().numpy()) for k, v in dev_res.items()}
         self._apply_nan_policy(self.results['flags'])
@@ -324,14 +330,14 @@ class BatchInversion:
             warnings.warn(msg, RuntimeWarning)
 
     def fit_gathered(self, n_total, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), group=None, batch_size=None,
-                     autocorr=False, rtd=False, model_curves=False):
+                     autocorr=False, rtd=False, model_curves=False, waic=False):
         """``fit`` for a shard-local inversion inside a ``torch.distributed`` job: this object holds spectra
         ``[spectrum_offset, spectrum_offset + n_spectra)`` of a survey of ``n_total`` sharded by ``shard_range``; after
         sampling, the summaries of all ranks are all-gathered (one NCCL collective) and the COMPLETE result
         (``n_total`` rows, host arrays) is returned on every rank.  Without a process group it equals ``fit``."""
         import torch.distributed as dist
         dev_res = self.fit_device(p0, discard, thin, percentiles, False, batch_size, autocorr=autocorr, rtd=rtd,
-                                  model_curves=model_curves)
+                                  model_curves=model_curves, waic=waic)
         if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
             dev_res = gather_packed(dev_res, int(n_total), dist.get_rank(group), dist.get_world_size(group), group)
         self.percentiles = tuple(float(q) for q in percentiles)
@@ -340,7 +346,7 @@ class BatchInversion:
         return self.results
 
     def fit_device(self, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), keep_chain=False,
-                   batch_size=None, _chain_to_host=False, autocorr=False, rtd=False, model_curves=False):
+                   batch_size=None, _chain_to_host=False, autocorr=False, rtd=False, model_curves=False, waic=False):
         """Same as ``fit`` but leaves the summaries on the GPU (for the NCCL gather).  With ``keep_chain`` the kept
         chains of all sub-batches stay on the device too (``fit`` moves each sub-batch's chain to the host instead)."""
         if rtd and self.model != 'decomp':
@@ -366,6 +372,10 @@ class BatchInversion:
                            total_chargeability_std=torch.empty((0,), **f64))
             if model_curves:
                 out['model_percentiles'] = torch.empty((0, P, 2, self.w.shape[-1]), **f64)
+            if waic:
+                out.update(elpd_waic=torch.empty((0,), **f64), p_waic=torch.empty((0,), **f64),
+                           se_elpd_waic=torch.empty((0,), **f64), waic_pointwise=torch.empty((0, self.w.shape[-1]), **f64),
+                           waic_n_high_p=torch.empty((0,), dtype=torch.int32, device=self.device))
             if keep_chain:
                 out['chain'], out['log_prob'] = torch.empty((0, nk, W, ndim), **f64), torch.empty((0, nk, W), **f64)
                 if _chain_to_host:
@@ -384,6 +394,9 @@ class BatchInversion:
                 acc[k] = []
         if model_curves:
             acc['model_percentiles'] = []
+        if waic:
+            for k in ('elpd_waic', 'p_waic', 'se_elpd_waic', 'waic_pointwise', 'waic_n_high_p'):
+                acc[k] = []
         if keep_chain:
             acc['chain'], acc['log_prob'] = [], []
         for lo in range(0, B, bs):
@@ -421,6 +434,13 @@ class BatchInversion:
                 acc['total_chargeability_std'].append(rs['std'][:, S])
             if model_curves:
                 acc['model_percentiles'].append(self._model_curves(spec, flat, w, percentiles))
+            if waic:
+                wa = engine.waic(spec, flat, w, y, ye)
+                acc['elpd_waic'].append(wa['elpd'])
+                acc['p_waic'].append(wa['p_waic'])
+                acc['se_elpd_waic'].append(wa['se'])
+                acc['waic_pointwise'].append(wa['lppd'] - wa['p'])
+                acc['waic_n_high_p'].append(wa['n_high_p'])
             acc['acceptance_fraction'].append(res['accepted'].to(torch.float64).mean(1) / float(self.nsteps))
             acc['flags'].append(res['flags'])
             if keep_chain and _chain_to_host:      # sub-batching stays effective: nothing accumulates on the device

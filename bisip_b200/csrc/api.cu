@@ -11,6 +11,7 @@
 #include "model_pct.cuh"
 #include "autocorr.cuh"
 #include "rtd_stats.cuh"
+#include "waic.cuh"
 
 namespace bisip {
 
@@ -310,24 +311,30 @@ int bisip_column_stats(const double* data, int n_spectra, int64_t n_samples, int
   return BISIP_OK;
 }
 
+// model description of the kernels built on model_points (model_pct.cuh): the decomposition runs its collapsed FP64
+// column form for every precision, and the loops over modes / coefficients do not have the sampler kernels' tile limits
+static int check_point_desc(const bisip_model_desc* desc, bisip_model_desc* out, const char* name) {
+  if (!desc) return fail(BISIP_ERR_BAD_ARG, "desc is null");
+  bisip_model_desc d = *desc;
+  if (d.model == BISIP_MODEL_DECOMP) d.precision = BISIP_PREC_FP64_COLLAPSED;   // the column form; FP64 for every mode
+  bisip_model_desc chk = d;
+  if (chk.model == BISIP_MODEL_COLECOLE && chk.n_modes > kMaxModes) { chk.n_modes = 1; chk.ndim = 4; }
+  if (chk.model == BISIP_MODEL_DECOMP && chk.n_coef > 8) { chk.n_coef = 8; chk.ndim = 9; chk.precision = BISIP_PREC_FP64; }
+  if (int rc = check_desc(&chk)) return rc;
+  if (d.model == BISIP_MODEL_COLECOLE && (d.n_modes < 1 || d.ndim != 1 + 3 * d.n_modes))
+    return fail(BISIP_ERR_BAD_ARG, "ColeCole ndim != 1+3*n_modes");
+  if (d.model == BISIP_MODEL_DECOMP && (d.ndim != 1 + d.n_coef || d.n_coef > kMaxCoefPct))
+    return fail(d.n_coef > kMaxCoefPct ? BISIP_ERR_UNSUPPORTED : BISIP_ERR_BAD_ARG, std::string(name) + ": bad n_coef");
+  *out = d;
+  return BISIP_OK;
+}
+
 int bisip_model_percentile(const bisip_model_desc* desc, int n_spectra, int64_t n_theta, const double* theta,
                            const double* w, int64_t w_stride, const double* taus, const double* log_taus,
                            int64_t tau_stride, int n_pct, const int64_t* pct_lo, const double* pct_gamma,
                            double* pct_out, void* stream) {
-  if (!desc) return fail(BISIP_ERR_BAD_ARG, "desc is null");
-  bisip_model_desc d = *desc;
-  if (d.model == BISIP_MODEL_DECOMP) d.precision = BISIP_PREC_FP64_COLLAPSED;   // the column form; FP64 for every mode
-  {
-    // this kernel loops over modes / coefficients: the tile-shaped limits of the sampler kernels do not apply
-    bisip_model_desc chk = d;
-    if (chk.model == BISIP_MODEL_COLECOLE && chk.n_modes > kMaxModes) { chk.n_modes = 1; chk.ndim = 4; }
-    if (chk.model == BISIP_MODEL_DECOMP && chk.n_coef > 8) { chk.n_coef = 8; chk.ndim = 9; chk.precision = BISIP_PREC_FP64; }
-    if (int rc = check_desc(&chk)) return rc;
-    if (d.model == BISIP_MODEL_COLECOLE && (d.n_modes < 1 || d.ndim != 1 + 3 * d.n_modes))
-      return fail(BISIP_ERR_BAD_ARG, "ColeCole ndim != 1+3*n_modes");
-    if (d.model == BISIP_MODEL_DECOMP && (d.ndim != 1 + d.n_coef || d.n_coef > kMaxCoefPct))
-      return fail(d.n_coef > kMaxCoefPct ? BISIP_ERR_UNSUPPORTED : BISIP_ERR_BAD_ARG, "bisip_model_percentile: bad n_coef");
-  }
+  bisip_model_desc d;
+  if (int rc = check_point_desc(desc, &d, "bisip_model_percentile")) return rc;
   if (n_spectra <= 0 || n_theta <= 0 || !theta || !w || n_pct <= 0 || !pct_lo || !pct_gamma || !pct_out)
     return fail(BISIP_ERR_BAD_ARG, "bisip_model_percentile: bad argument");
   if (d.model == BISIP_MODEL_DECOMP && (!taus || !log_taus)) return fail(BISIP_ERR_BAD_ARG, "bisip_model_percentile: taus/log_taus null");
@@ -396,6 +403,33 @@ int bisip_rtd_stats(int n_spectra, int64_t n_samples, int ndim, int n_coef, int 
   if (stats_fits_smem(n_samples, 2 * n_pct, &smem))
     return launch(rtd_stats_smem_kernel, grid, smem, (cudaStream_t)stream, "rtd_stats", &P, kStatThreads);
   return launch(rtd_stats_global_kernel, grid, 0, (cudaStream_t)stream, "rtd_stats", &P, kThreads);
+}
+
+int bisip_waic(const bisip_model_desc* desc, int n_spectra, int64_t n_theta, const double* theta, const double* w,
+               int64_t w_stride, const double* taus, const double* log_taus, int64_t tau_stride, const double* y,
+               const double* yerr, double* lppd_out, double* p_out, double* elpd_out, double* p_waic_out,
+               double* se_out, int32_t* n_high_p_out, void* stream) {
+  bisip_model_desc d;
+  if (int rc = check_point_desc(desc, &d, "bisip_waic")) return rc;
+  if (n_spectra <= 0 || n_theta < 2 || !theta || !w || w_stride < 0 || tau_stride < 0 || !y || !yerr || !lppd_out ||
+      !p_out || !elpd_out || !p_waic_out || !se_out || !n_high_p_out)
+    return fail(BISIP_ERR_BAD_ARG, "bisip_waic: bad argument");
+  if (d.model == BISIP_MODEL_DECOMP && (!taus || !log_taus)) return fail(BISIP_ERR_BAD_ARG, "bisip_waic: taus/log_taus null");
+  if (n_spectra > 65535) return fail(BISIP_ERR_UNSUPPORTED, "bisip_waic: n_spectra > 65535 per call");
+  DeviceGuard guard(theta);
+  WaicParams P;
+  P.d = d; P.n = n_theta; P.theta = theta; P.w = w; P.w_stride = w_stride;
+  P.taus = taus; P.log_taus = log_taus; P.tau_stride = tau_stride; P.y = y; P.yerr = yerr;
+  P.lppd_out = lppd_out; P.p_out = p_out; P.elpd_out = elpd_out; P.p_waic_out = p_waic_out; P.se_out = se_out;
+  P.n_high_p_out = n_high_p_out;
+  const dim3 grid(n_spectra);
+  const cudaStream_t st = (cudaStream_t)stream;
+  switch (d.model) {
+    case BISIP_MODEL_DECOMP: return launch(waic_kernel<BISIP_MODEL_DECOMP>, grid, 0, st, "waic", &P, kWaicThreads);
+    case BISIP_MODEL_COLECOLE: return launch(waic_kernel<BISIP_MODEL_COLECOLE>, grid, 0, st, "waic", &P, kWaicThreads);
+    case BISIP_MODEL_DIAS: return launch(waic_kernel<BISIP_MODEL_DIAS>, grid, 0, st, "waic", &P, kWaicThreads);
+    default: return launch(waic_kernel<BISIP_MODEL_SHIN>, grid, 0, st, "waic", &P, kWaicThreads);
+  }
 }
 
 }  // extern "C"

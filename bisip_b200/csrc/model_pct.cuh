@@ -50,11 +50,70 @@ __device__ __forceinline__ void colecole_point(const double* __restrict__ th, in
   zim = -R0 * sim;
 }
 
+// Z of one parameter vector at F frequencies, FP64, real and imaginary part together: the per-sample evaluation of
+// model_percentile_kernel (F = 1) and waic_kernel (waic.cuh).
+//   decomposition: the collapsed column form z_c = R0 delta_c - sum_i (R0 a_i) G_ic, accumulated in ascending i (the
+//     arithmetic of decomp_c_eval_Z); g[i * 2F + f] is G_i of frequency f's real part, g[i * 2F + F + f] its imaginary part
+//   Cole-Cole / Dias / Shin: fq + f * kFq is frequency f's record ([0] w, [1] sqrt(w), [2] ln(w)), evaluated as the
+//     batched forward kernels (FAST = false); the theta-only constants of Dias / Shin are prepared once for all F
+template <int F>
+__device__ __forceinline__ void model_points(const bisip_model_desc& d, const double* __restrict__ th,
+                                             const double* __restrict__ g, const double* __restrict__ fq,
+                                             double (&zre)[F], double (&zim)[F]) {
+  switch (d.model) {
+    case BISIP_MODEL_DECOMP: {
+      const double R0 = th[0];
+      double are[F], aim[F];
+#pragma unroll
+      for (int f = 0; f < F; ++f) are[f] = aim[f] = 0.0;
+#pragma unroll 1
+      for (int q = 0; q < d.n_coef; ++q) {
+        const double cq = R0 * th[1 + q];
+        const double* gq = g + q * 2 * F;
+#pragma unroll
+        for (int f = 0; f < F; ++f) {
+          are[f] = fma(cq, gq[f], are[f]);
+          aim[f] = fma(cq, gq[F + f], aim[f]);
+        }
+      }
+#pragma unroll
+      for (int f = 0; f < F; ++f) {
+        zre[f] = R0 - are[f];
+        zim[f] = 0.0 - aim[f];                          // delta_c = 0: the sign of a zero as decomp_c_eval_Z
+      }
+      break;
+    }
+    case BISIP_MODEL_COLECOLE:
+#pragma unroll
+      for (int f = 0; f < F; ++f) colecole_point(th, d.n_modes, fq[f * kFq + 2], zre[f], zim[f]);
+      break;
+    case BISIP_MODEL_DIAS: {
+      double rc[DiasRow::kRC];
+      DiasRow::prepare(th, 0, rc);
+      DiasRow rr;
+      rr.R0 = rc[0]; rr.R0m = rc[1]; rr.tau = rc[2]; rr.tau_p = rc[3]; rr.sfac = rc[4];
+#pragma unroll
+      for (int f = 0; f < F; ++f) rr.eval<false>(fq + f * kFq, zre[f], zim[f]);
+      break;
+    }
+    default: {
+      double rc[ShinRow::kRC];
+      ShinRow::prepare(th, 0, rc);
+      ShinRow rr;
+#pragma unroll
+      for (int e = 0; e < 2; ++e) { rr.iR[e] = rc[4 * e]; rr.n[e] = rc[4 * e + 1]; rr.qc[e] = rc[4 * e + 2]; rr.qs[e] = rc[4 * e + 3]; }
+#pragma unroll
+      for (int f = 0; f < F; ++f) rr.eval<false>(fq + f * kFq, zre[f], zim[f]);
+      break;
+    }
+  }
+}
+
 // grid (2N, B), kStatThreads threads, dynamic shared memory stats_smem_bytes(n, 2 npct)
 __global__ void __launch_bounds__(kStatThreads, 1) model_percentile_kernel(const ModelPctParams P) {
   extern __shared__ __align__(16) unsigned char stats_dyn[];
   __shared__ double red[32];
-  __shared__ double s_g[kMaxCoefPct];
+  __shared__ double s_g[2 * kMaxCoefPct];
   __shared__ __align__(16) double s_fq[kFq];
   constexpr int NT = kStatThreads;
   const int c = blockIdx.x, b = blockIdx.y, tid = threadIdx.x;
@@ -72,10 +131,10 @@ __global__ void __launch_bounds__(kStatThreads, 1) model_percentile_kernel(const
     const int D = P.d.n_coef, S = P.d.n_tau;
     const double* taus = P.taus + (size_t)b * P.tau_stride;
     const double* lts = P.log_taus + (size_t)b * P.tau_stride * D;
-    if (tid < D) {
+    if (tid < 2 * D) {                              // s_g[2 q + part], the layout of model_points<1>
       double cs, sn;
       sincospi(0.5 * P.d.c_exp, &sn, &cs);
-      s_g[tid] = dot2_lk(lts + (size_t)tid * S, taus, S, wj, P.d.c_exp, cs, sn, imag, 1.0);
+      s_g[tid] = dot2_lk(lts + (size_t)(tid >> 1) * S, taus, S, wj, P.d.c_exp, cs, sn, (tid & 1) != 0, 1.0);
     }
   } else if (tid == 0) {
     s_fq[0] = wj; s_fq[1] = sqrt(wj); s_fq[2] = log(wj); s_fq[3] = 0.0;
@@ -87,37 +146,9 @@ __global__ void __launch_bounds__(kStatThreads, 1) model_percentile_kernel(const
   int nan = 0;
   for (int i = tid; i < n; i += NT) {
     const double* th = theta + (size_t)i * ndim;
-    double zre, zim;
-    switch (P.d.model) {
-      case BISIP_MODEL_DECOMP: {
-        const double R0 = th[0];
-        double acc = 0.0;
-        for (int q = 0; q < P.d.n_coef; ++q) acc = fma(R0 * th[1 + q], s_g[q], acc);
-        zre = zim = (imag ? 0.0 : R0) - acc;           // decomp_c_eval_Z: R0 * delta_c - acc
-        break;
-      }
-      case BISIP_MODEL_COLECOLE:
-        colecole_point(th, P.d.n_modes, s_fq[2], zre, zim);
-        break;
-      case BISIP_MODEL_DIAS: {
-        double rc[DiasRow::kRC];
-        DiasRow::prepare(th, 0, rc);
-        DiasRow rr;
-        rr.R0 = rc[0]; rr.R0m = rc[1]; rr.tau = rc[2]; rr.tau_p = rc[3]; rr.sfac = rc[4];
-        rr.eval<false>(s_fq, zre, zim);
-        break;
-      }
-      default: {
-        double rc[ShinRow::kRC];
-        ShinRow::prepare(th, 0, rc);
-        ShinRow rr;
-#pragma unroll
-        for (int e = 0; e < 2; ++e) { rr.iR[e] = rc[4 * e]; rr.n[e] = rc[4 * e + 1]; rr.qc[e] = rc[4 * e + 2]; rr.qs[e] = rc[4 * e + 3]; }
-        rr.eval<false>(s_fq, zre, zim);
-        break;
-      }
-    }
-    const double v = imag ? zim : zre;
+    double zre[1], zim[1];
+    model_points<1>(P.d, th, s_g, s_fq, zre, zim);
+    const double v = imag ? zim[0] : zre[0];
     vals[i] = v;
     s += v;
     mn = fmin(mn, v);

@@ -281,3 +281,36 @@ def model_percentile(spec, theta, w, p):
         if k != npct:
             out[:, s0:s0 + k] = part
     return out
+
+
+def waic(spec, theta, w, y, yerr):
+    """WAIC of every spectrum from parameter vectors (``bisip_waic``; ``theta`` is read in place): theta (B, n, ndim)
+    with n >= 2, w (N,) or (B, N), y, yerr (B, 2, N) -> dict of ``lppd``, ``p`` (B, N), ``elpd``, ``p_waic``, ``se``
+    (B,) float64 and ``n_high_p`` (B,) int32.  With ll[s, j] the Gaussian log-likelihood of sample s at frequency j
+    (real and imaginary part together, with the reference's 2 ln sigma^2 term): lppd[j] = logsumexp_s ll - ln n,
+    p[j] = var_s(ll, ddof=1), elpd = sum_j (lppd - p), p_waic = sum_j p, se = sqrt(N var_j(lppd - p, ddof=1)),
+    n_high_p = #{j : p[j] > 0.4}.  Z in FP64 for every ``precision``; a NaN sample makes its spectrum all-NaN."""
+    lib = _lib.load()
+    _chk_cuda_f64(theta, w, y, yerr, spec.taus, spec.log_taus)
+    B, n, ndim = theta.shape
+    N = w.shape[-1]
+    if ndim != spec.ndim or tuple(y.shape) != (B, 2, N) or tuple(yerr.shape) != (B, 2, N):
+        raise ValueError(f"waic: theta (B, n, {spec.ndim}) and y, yerr (B, 2, {N}) expected")
+    dev = theta.device
+    f64 = dict(dtype=torch.float64, device=dev)
+    out = dict(lppd=torch.empty((B, N), **f64), p=torch.empty((B, N), **f64), elpd=torch.empty((B,), **f64),
+               p_waic=torch.empty((B,), **f64), se=torch.empty((B,), **f64),
+               n_high_p=torch.empty((B,), dtype=torch.int32, device=dev))
+    d = spec.desc(N)
+    ts = spec.tau_stride()
+    for s0 in range(0, B, 65535):                  # one launch per 65,535 spectra
+        k = min(65535, B - s0)
+        sl = slice(s0, s0 + k)
+        taus = spec.taus if ts == 0 else spec.taus[sl]
+        lts = spec.log_taus if ts == 0 else spec.log_taus[sl]
+        rc = lib.bisip_waic(C.byref(d), k, n, _lib.ptr(theta[sl]), _lib.ptr(w if w.dim() == 1 else w[sl]), _w_stride(w),
+                            _lib.ptr(taus), _lib.ptr(lts), ts, _lib.ptr(y[sl]), _lib.ptr(yerr[sl]),
+                            *[_lib.ptr(out[key][sl]) for key in ('lppd', 'p', 'elpd', 'p_waic', 'se', 'n_high_p')],
+                            _lib.stream_ptr(dev))
+        _lib.check(rc, "bisip_waic")
+    return out

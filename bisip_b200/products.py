@@ -53,7 +53,8 @@ def batch_table(param_names, results, ids=None, percentiles=(2.5, 50, 97.5)):
     id, acceptance fraction, flags, then mean / std / each percentile of every parameter, and — when the results hold
     ``autocorr_time`` (``fit(..., autocorr=True)``) — one ``<name>_tau`` column per parameter, then — when they hold the
     total chargeability (``fit(..., rtd=True)``) — ``total_m_mean``, ``total_m_std`` and one ``total_m_p<q>`` per
-    percentile.  The RTD and model-curve arrays stay in ``results``."""
+    percentile, then — when they hold the WAIC (``fit(..., waic=True)``) — ``elpd_waic``, ``p_waic``, ``se_elpd_waic``
+    and ``waic_n_high_p``.  The RTD, model-curve and pointwise WAIC arrays stay in ``results``."""
     B = results['mean'].shape[0]
     ids = np.arange(B) if ids is None else np.asarray(ids)
     cols = ['spectrum', 'acceptance_fraction', 'flags']
@@ -72,4 +73,26 @@ def batch_table(param_names, results, ids=None, percentiles=(2.5, 50, 97.5)):
         cols += ['total_m_mean', 'total_m_std'] + [f'total_m_p{q:g}' for q in percentiles]
         blocks += [results['total_chargeability_mean'][:, None], results['total_chargeability_std'][:, None],
                    results['total_chargeability_percentiles']]
+    if 'elpd_waic' in results:
+        cols += ['elpd_waic', 'p_waic', 'se_elpd_waic', 'waic_n_high_p']
+        blocks += [results['elpd_waic'][:, None], results['p_waic'][:, None], results['se_elpd_waic'][:, None],
+                   results['waic_n_high_p'].astype(np.float64)[:, None]]
     return cols, np.concatenate(blocks, axis=1)
+
+
+def compare_waic(res_a, res_b):
+    """Spectrum-by-spectrum WAIC comparison of two fits (``fit(..., waic=True)`` results, or ``get_waic`` dicts):
+    ``elpd_diff`` = elpd_waic_a - elpd_waic_b (positive: model a is expected to predict the data better) and
+    ``se_diff`` = sqrt(N var_j(pointwise_a - pointwise_b, ddof=1)), the standard error of that difference (Vehtari,
+    Gelman & Gabry 2017), each of shape (B,) (scalars for single-spectrum dicts).  The comparison is only meaningful for
+    two fits of the same ``zn`` / ``zn_err``: the pointwise terms are paired by frequency.  Raises ``ValueError`` when
+    the shapes differ."""
+    ea, eb = np.asarray(res_a['elpd_waic'], dtype=np.float64), np.asarray(res_b['elpd_waic'], dtype=np.float64)
+    pa = np.asarray(res_a['waic_pointwise'], dtype=np.float64)
+    pb = np.asarray(res_b['waic_pointwise'], dtype=np.float64)
+    if ea.shape != eb.shape or pa.shape != pb.shape or pa.shape[:-1] != ea.shape:
+        raise ValueError(f"compare_waic: shapes differ (elpd_waic {ea.shape} vs {eb.shape}, "
+                         f"waic_pointwise {pa.shape} vs {pb.shape})")
+    d = pa - pb
+    N = d.shape[-1]
+    return {'elpd_diff': ea - eb, 'se_diff': np.sqrt(N * np.var(d, axis=-1, ddof=1))}

@@ -35,6 +35,22 @@ class utils(object):
         res = out[0].cpu().numpy()
         return res if np.ndim(p) else res[0]
 
+    def get_waic(self, chain=None, **kwargs):
+        """WAIC of the fit over an MCMC chain (Watanabe's widely applicable information criterion, as in Vehtari,
+        Gelman & Gabry 2017), for comparing models fitted to the same data: a dict of ``elpd_waic``, ``p_waic``,
+        ``se_elpd_waic`` (floats), ``waic_pointwise`` (N,) = lppd - p per frequency and ``waic_n_high_p`` (the number
+        of frequencies with p > 0.4).  The kernel behind ``BatchInversion.fit(..., waic=True)`` (``engine.waic``), FP64
+        for every precision.  ``chain`` / ``discard`` / ``thin`` as in ``get_model_percentile``."""
+        chain = self.parse_chain(chain, **kwargs)
+        dev = _lib.require_cuda(getattr(self, "device", None))
+        th = _lib.dev_f64(chain, dev).reshape(1, -1, chain.shape[-1])
+        w = _lib.dev_const(self.data['w'], dev)
+        y = _lib.dev_f64(self.data['zn'], dev).reshape(1, 2, -1)
+        ye = _lib.dev_f64(self.data['zn_err'], dev).reshape(1, 2, -1)
+        r = {k: v[0].cpu().numpy() for k, v in engine.waic(self._spec(dev), th, w, y, ye).items()}
+        return {'elpd_waic': float(r['elpd']), 'p_waic': float(r['p_waic']), 'se_elpd_waic': float(r['se']),
+                'waic_pointwise': r['lppd'] - r['p'], 'waic_n_high_p': int(r['n_high_p'])}
+
     # ---------------------------------------------------------------- parameter statistics
     def _chain_stats(self, chain, p=None, mean=False, std=False):
         dev = _lib.require_cuda(getattr(self, "device", None))

@@ -25,6 +25,7 @@
  *                               sampler.get_autocorr_time (models.py:154-159)
  *   bisip_rtd_stats          <- relaxation_time_distribution / total_m of decomposition.ipynb
  *                               cells 25-29 over the chain, then np.percentile / mean / std
+ *   bisip_waic               <- (no counterpart: the tutorials compare models by eye with plot_fit)
  *
  * Layouts (all row-major, float64):
  *   theta   [n_spectra][n_theta][ndim]      parameter vectors (order as the reference's
@@ -235,6 +236,29 @@ int bisip_rtd_stats(int n_spectra, int64_t n_samples, int ndim, int n_coef, int 
                     const double *theta, const double *log_taus, int64_t tau_stride,
                     int n_pct, const int64_t *pct_lo, const double *pct_gamma,
                     double *pct_out, double *mean_out, double *std_out, void *stream);
+
+/*
+ * WAIC (Watanabe's widely applicable information criterion, as in Vehtari, Gelman & Gabry 2017) of every spectrum
+ * from its chain, read in place, for comparing two models fitted to the same data.
+ *   theta [n_spectra][n_theta][ndim] (n_theta >= 2), w / taus / log_taus as in bisip_forward, y / yerr [n_spectra][2][N]
+ * One data point per frequency j (its real and imaginary part are one measurement):
+ *   ll[s][j] = -0.5 sum_{p in re, im} ((y[p][j] - Z[p][j](theta_s))^2 / yerr[p][j]^2 + 2 ln yerr[p][j]^2)
+ * (sum_j ll[s][j] is the reference's _log_likelihood, models.py:59-62), and
+ *   lppd_out[b][j] = logsumexp_s ll[s][j] - ln n_theta        p_out[b][j] = var_s(ll[s][j], ddof=1)
+ *   elpd_out[b]    = sum_j (lppd - p)                          p_waic_out[b] = sum_j p
+ *   se_out[b]      = sqrt(N var_j(lppd - p, ddof=1))           n_high_p_out[b] = #{j : p[j] > 0.4}  (int32)
+ * Z is evaluated in FP64 for every desc->precision (the decomposition in its collapsed column form, as
+ * bisip_model_percentile).  A NaN anywhere in a spectrum's samples makes all its outputs NaN (n_high_p 0).  One launch,
+ * one CTA per spectrum; fixed-order reductions: a spectrum's result depends on its own chain and data only.  No
+ * workspace and no limit on n_theta.
+ * BISIP_ERR_BAD_ARG: null pointer, non-positive size, n_theta < 2, bad ndim / n_coef, w_stride or tau_stride < 0;
+ * BISIP_ERR_UNSUPPORTED: n_spectra > 65535, n_coef > 32.
+ */
+int bisip_waic(const bisip_model_desc *desc, int n_spectra, int64_t n_theta, const double *theta,
+               const double *w, int64_t w_stride, const double *taus, const double *log_taus, int64_t tau_stride,
+               const double *y, const double *yerr,
+               double *lppd_out, double *p_out, double *elpd_out, double *p_waic_out, double *se_out,
+               int32_t *n_high_p_out, void *stream);
 
 #ifdef __cplusplus
 }
