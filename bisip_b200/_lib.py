@@ -24,7 +24,7 @@ EXPORTS = ("bisip_abi_version", "bisip_last_error", "bisip_launch_count", "bisip
            "bisip_log_probability", "bisip_decomp_build_kernel", "bisip_n_keep",
            "bisip_ensemble_run", "bisip_column_stats_workspace", "bisip_column_stats",
            "bisip_decomp_kernel_kind", "bisip_model_percentile", "bisip_gauss_loglike",
-           "bisip_autocorr_time", "bisip_rtd_stats", "bisip_waic")
+           "bisip_autocorr_time", "bisip_rtd_stats", "bisip_waic", "bisip_psis_loo")
 KERNEL_KINDS = {0: "dmma", 1: "dmma-cluster", 2: "mma-tf32", 3: "tcgen05", 4: "tcgen05-cluster", 5: "fp64-collapsed"}
 
 
@@ -88,6 +88,9 @@ def load():
     lib.bisip_waic.restype = C.c_int
     lib.bisip_waic.argtypes = [C.POINTER(ModelDesc), i32, i64, vp, vp, i64, vp, vp, i64, vp, vp, vp, vp, vp, vp, vp,
                                vp, vp]
+    lib.bisip_psis_loo.restype = C.c_int
+    lib.bisip_psis_loo.argtypes = [C.POINTER(ModelDesc), i32, i64, vp, vp, i64, vp, vp, i64, vp, vp, vp, vp, vp, vp, vp,
+                                   vp, vp, vp]
     if lib.bisip_abi_version() != ABI_VERSION:
         raise BisipError("libbisip_b200.so ABI version mismatch")
     _lib = lib

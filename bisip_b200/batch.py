@@ -133,7 +133,8 @@ def gather_chain_to_rank0(chain, n_total, rank, world, group=None, chunk_bytes=1
 
 
 def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 97.5), p0=None, gather_chain=False,
-                group=None, batch_size=None, autocorr=False, rtd=False, model_curves=False, waic=False, **kwargs):
+                group=None, batch_size=None, autocorr=False, rtd=False, model_curves=False, waic=False, loo=False,
+                **kwargs):
     """Invert a whole survey on all ranks of the current ``torch.distributed`` job (one process per GPU).
 
     The reference inverts a batch as a serial loop over files (``docs/tutorials/decomposition.ipynb`` cells 9-10);
@@ -143,7 +144,8 @@ def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 9
     per-spectrum summaries are all-gathered with one NCCL collective, so every rank returns the complete result:
     ``percentiles`` (B, len(p), ndim), ``mean``, ``std`` (B, ndim), ``acceptance_fraction``, ``flags`` (B,), with
     ``autocorr=True`` ``autocorr_time`` (B, ndim), with ``rtd=True`` / ``model_curves=True`` the RTD,
-    total-chargeability and model-curve keys, and with ``waic=True`` the WAIC keys (see ``BatchInversion.fit``).  With ``gather_chain=True`` the kept
+    total-chargeability and model-curve keys, with ``waic=True`` the WAIC keys and with ``loo=True`` the PSIS-LOO keys
+    (see ``BatchInversion.fit``).  With ``gather_chain=True`` the kept
     chains (``discard`` / ``thin``) are gathered to rank 0 in chunks (``chain`` (B, n_keep, W, ndim) on rank 0, None
     elsewhere).  Without an initialised process group it runs the
     whole survey on the current device.  ``kwargs`` go to ``BatchInversion`` (nwalkers, nsteps, poly_deg, ...)."""
@@ -157,8 +159,8 @@ def fit_sharded(model, w, zn, zn_err, discard=0, thin=1, percentiles=(2.5, 50, 9
     inv = BatchInversion(model, w_arr if w_arr.ndim == 1 else w_arr[lo:hi], zn[lo:hi], zn_err[lo:hi],
                          spectrum_offset=lo + int(kwargs.pop('spectrum_offset', 0)), **kwargs)
     # the optional products are passed only when set, so fit_device overrides written for the older signature keep working
-    extra = {k: True for k, on in (('autocorr', autocorr), ('rtd', rtd), ('model_curves', model_curves), ('waic', waic))
-             if on}
+    extra = {k: True for k, on in (('autocorr', autocorr), ('rtd', rtd), ('model_curves', model_curves), ('waic', waic),
+                                   ('loo', loo)) if on}
     dev_res = inv.fit_device(None if p0 is None else p0[lo:hi], discard, thin, percentiles, gather_chain, batch_size,
                              **extra)
     chain = dev_res.pop('chain', None)
@@ -288,7 +290,7 @@ class BatchInversion:
 
     # ------------------------------------------------------------------ fit
     def fit(self, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), keep_chain=False, batch_size=None,
-            autocorr=False, rtd=False, model_curves=False, waic=False):
+            autocorr=False, rtd=False, model_curves=False, waic=False, loo=False):
         """Sample every spectrum and summarise the kept chain on the device.
 
         Returns (and stores in ``self.results``) a dict of host arrays:
@@ -311,9 +313,16 @@ class BatchInversion:
         data (``products.compare_waic``): ``elpd_waic``, ``p_waic``, ``se_elpd_waic`` (B,), ``waic_pointwise`` (B, N)
         = lppd - p per frequency, and ``waic_n_high_p`` (B,) int32, the number of frequencies with p > 0.4 (where WAIC
         is unreliable).  FP64 for every ``precision``; one launch per sub-batch.
+        With ``loo=True`` also PSIS-LOO, leave-one-out cross-validation by Pareto-smoothed importance sampling of every
+        spectrum over its flat chain (``engine.psis_loo``, as ArviZ's ``psislw`` with r_eff = 1; Vehtari, Gelman & Gabry
+        2017), the estimate their paper recommends where WAIC is unreliable (``products.compare_loo``): ``elpd_loo``,
+        ``p_loo``, ``se_elpd_loo`` (B,), ``loo_pointwise`` (B, N) = elpd_loo per frequency, ``pareto_k`` (B, N), the
+        Pareto shape of each frequency's importance ratios (large k: a measurement the posterior depends on heavily),
+        and ``loo_n_high_k`` (B,) int32, the number of frequencies with k > min(1 - 1/log10 S, 0.7) for S flat-chain
+        samples.  FP64 for every ``precision``; two launches per sub-batch.
         """
         dev_res = self.fit_device(p0, discard, thin, percentiles, keep_chain, batch_size, _chain_to_host=True,
-                                  autocorr=autocorr, rtd=rtd, model_curves=model_curves, waic=waic)
+                                  autocorr=autocorr, rtd=rtd, model_curves=model_curves, waic=waic, loo=loo)
         self.percentiles = tuple(float(q) for q in percentiles)
         self.results = {k: (v if isinstance(v, np.ndarray) else v.cpu().numpy()) for k, v in dev_res.items()}
         self._apply_nan_policy(self.results['flags'])
@@ -330,14 +339,14 @@ class BatchInversion:
             warnings.warn(msg, RuntimeWarning)
 
     def fit_gathered(self, n_total, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), group=None, batch_size=None,
-                     autocorr=False, rtd=False, model_curves=False, waic=False):
+                     autocorr=False, rtd=False, model_curves=False, waic=False, loo=False):
         """``fit`` for a shard-local inversion inside a ``torch.distributed`` job: this object holds spectra
         ``[spectrum_offset, spectrum_offset + n_spectra)`` of a survey of ``n_total`` sharded by ``shard_range``; after
         sampling, the summaries of all ranks are all-gathered (one NCCL collective) and the COMPLETE result
         (``n_total`` rows, host arrays) is returned on every rank.  Without a process group it equals ``fit``."""
         import torch.distributed as dist
         dev_res = self.fit_device(p0, discard, thin, percentiles, False, batch_size, autocorr=autocorr, rtd=rtd,
-                                  model_curves=model_curves, waic=waic)
+                                  model_curves=model_curves, waic=waic, loo=loo)
         if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
             dev_res = gather_packed(dev_res, int(n_total), dist.get_rank(group), dist.get_world_size(group), group)
         self.percentiles = tuple(float(q) for q in percentiles)
@@ -346,7 +355,8 @@ class BatchInversion:
         return self.results
 
     def fit_device(self, p0=None, discard=0, thin=1, percentiles=(2.5, 50, 97.5), keep_chain=False,
-                   batch_size=None, _chain_to_host=False, autocorr=False, rtd=False, model_curves=False, waic=False):
+                   batch_size=None, _chain_to_host=False, autocorr=False, rtd=False, model_curves=False, waic=False,
+                   loo=False):
         """Same as ``fit`` but leaves the summaries on the GPU (for the NCCL gather).  With ``keep_chain`` the kept
         chains of all sub-batches stay on the device too (``fit`` moves each sub-batch's chain to the host instead)."""
         if rtd and self.model != 'decomp':
@@ -376,6 +386,12 @@ class BatchInversion:
                 out.update(elpd_waic=torch.empty((0,), **f64), p_waic=torch.empty((0,), **f64),
                            se_elpd_waic=torch.empty((0,), **f64), waic_pointwise=torch.empty((0, self.w.shape[-1]), **f64),
                            waic_n_high_p=torch.empty((0,), dtype=torch.int32, device=self.device))
+            if loo:
+                N = self.w.shape[-1]
+                out.update(elpd_loo=torch.empty((0,), **f64), p_loo=torch.empty((0,), **f64),
+                           se_elpd_loo=torch.empty((0,), **f64), loo_pointwise=torch.empty((0, N), **f64),
+                           pareto_k=torch.empty((0, N), **f64),
+                           loo_n_high_k=torch.empty((0,), dtype=torch.int32, device=self.device))
             if keep_chain:
                 out['chain'], out['log_prob'] = torch.empty((0, nk, W, ndim), **f64), torch.empty((0, nk, W), **f64)
                 if _chain_to_host:
@@ -396,6 +412,9 @@ class BatchInversion:
             acc['model_percentiles'] = []
         if waic:
             for k in ('elpd_waic', 'p_waic', 'se_elpd_waic', 'waic_pointwise', 'waic_n_high_p'):
+                acc[k] = []
+        if loo:
+            for k in ('elpd_loo', 'p_loo', 'se_elpd_loo', 'loo_pointwise', 'pareto_k', 'loo_n_high_k'):
                 acc[k] = []
         if keep_chain:
             acc['chain'], acc['log_prob'] = [], []
@@ -441,6 +460,14 @@ class BatchInversion:
                 acc['se_elpd_waic'].append(wa['se'])
                 acc['waic_pointwise'].append(wa['lppd'] - wa['p'])
                 acc['waic_n_high_p'].append(wa['n_high_p'])
+            if loo:
+                ps = engine.psis_loo(spec, flat, w, y, ye)
+                acc['elpd_loo'].append(ps['elpd'])
+                acc['p_loo'].append(ps['p_loo'])
+                acc['se_elpd_loo'].append(ps['se'])
+                acc['loo_pointwise'].append(ps['elpd_i'])
+                acc['pareto_k'].append(ps['pareto_k'])
+                acc['loo_n_high_k'].append(ps['n_high_k'])
             acc['acceptance_fraction'].append(res['accepted'].to(torch.float64).mean(1) / float(self.nsteps))
             acc['flags'].append(res['flags'])
             if keep_chain and _chain_to_host:      # sub-batching stays effective: nothing accumulates on the device

@@ -12,6 +12,7 @@
 #include "autocorr.cuh"
 #include "rtd_stats.cuh"
 #include "waic.cuh"
+#include "loo.cuh"
 
 namespace bisip {
 
@@ -111,6 +112,14 @@ __global__ void gauss_loglike_kernel(const double* __restrict__ Z, const double*
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
   if (lane == 0) out[row] = -0.5 * acc;
+}
+
+// bisip_psis_loo: loo_kernel of one model, the column in shared memory or recomputed per pass
+template <int MODEL>
+int launch_loo(const LooParams& P, bool smem_path, size_t smem, cudaStream_t st) {
+  const dim3 grid(P.d.n_freq, P.B);
+  return smem_path ? launch(loo_kernel<MODEL, true>, grid, smem, st, "psis_loo", &P, kStatThreads)
+                   : launch(loo_kernel<MODEL, false>, grid, smem, st, "psis_loo", &P, kThreads);
 }
 
 }  // namespace
@@ -430,6 +439,44 @@ int bisip_waic(const bisip_model_desc* desc, int n_spectra, int64_t n_theta, con
     case BISIP_MODEL_DIAS: return launch(waic_kernel<BISIP_MODEL_DIAS>, grid, 0, st, "waic", &P, kWaicThreads);
     default: return launch(waic_kernel<BISIP_MODEL_SHIN>, grid, 0, st, "waic", &P, kWaicThreads);
   }
+}
+
+int bisip_psis_loo(const bisip_model_desc* desc, int n_spectra, int64_t n_theta, const double* theta, const double* w,
+                   int64_t w_stride, const double* taus, const double* log_taus, int64_t tau_stride, const double* y,
+                   const double* yerr, double* elpd_i_out, double* p_i_out, double* k_out, double* elpd_out,
+                   double* p_loo_out, double* se_out, int32_t* n_high_k_out, void* stream) {
+  bisip_model_desc d;
+  if (int rc = check_point_desc(desc, &d, "bisip_psis_loo")) return rc;
+  if (n_spectra <= 0 || n_theta < 2 || !theta || !w || w_stride < 0 || tau_stride < 0 || !y || !yerr || !elpd_i_out ||
+      !p_i_out || !k_out || !elpd_out || !p_loo_out || !se_out || !n_high_k_out)
+    return fail(BISIP_ERR_BAD_ARG, "bisip_psis_loo: bad argument");
+  if (d.model == BISIP_MODEL_DECOMP && (!taus || !log_taus)) return fail(BISIP_ERR_BAD_ARG, "bisip_psis_loo: taus/log_taus null");
+  if (n_spectra > 65535) return fail(BISIP_ERR_UNSUPPORTED, "bisip_psis_loo: n_spectra > 65535 per call");
+  DeviceGuard guard(theta);
+  const size_t optin = (size_t)device_smem_optin();
+  // the ll column in shared memory when it fits, else recomputed per pass with only the tail buffer in shared memory
+  size_t smem = loo_smem_bytes(n_theta);
+  const bool smem_path = n_theta <= 0x7fffffff / 8 && smem + kStatStaticSmem <= optin;
+  if (!smem_path) {
+    smem = std::max(loo_tail_bytes(n_theta), (size_t)256 * 4);   // and the radix select's histogram before it
+    if (smem + kStatStaticSmem > optin)
+      return fail(BISIP_ERR_UNSUPPORTED, "bisip_psis_loo: the Pareto tail of the chain does not fit in shared memory");
+  }
+  LooParams P;
+  P.d = d; P.n = n_theta; P.B = n_spectra; P.theta = theta; P.w = w; P.w_stride = w_stride;
+  P.taus = taus; P.log_taus = log_taus; P.tau_stride = tau_stride; P.y = y; P.yerr = yerr;
+  P.elpd_i_out = elpd_i_out; P.p_i_out = p_i_out; P.k_out = k_out;
+  P.elpd_out = elpd_out; P.p_loo_out = p_loo_out; P.se_out = se_out; P.n_high_k_out = n_high_k_out;
+  const cudaStream_t st = (cudaStream_t)stream;
+  int rc;
+  switch (d.model) {
+    case BISIP_MODEL_DECOMP: rc = launch_loo<BISIP_MODEL_DECOMP>(P, smem_path, smem, st); break;
+    case BISIP_MODEL_COLECOLE: rc = launch_loo<BISIP_MODEL_COLECOLE>(P, smem_path, smem, st); break;
+    case BISIP_MODEL_DIAS: rc = launch_loo<BISIP_MODEL_DIAS>(P, smem_path, smem, st); break;
+    default: rc = launch_loo<BISIP_MODEL_SHIN>(P, smem_path, smem, st); break;
+  }
+  if (rc) return rc;
+  return launch(loo_totals_kernel, dim3((n_spectra + 127) / 128), 0, st, "psis_loo_totals", &P, 128);
 }
 
 }  // extern "C"

@@ -314,3 +314,40 @@ def waic(spec, theta, w, y, yerr):
                             _lib.stream_ptr(dev))
         _lib.check(rc, "bisip_waic")
     return out
+
+
+def psis_loo(spec, theta, w, y, yerr):
+    """PSIS-LOO of every spectrum from parameter vectors (``bisip_psis_loo``; ``theta`` is read in place): leave-one-out
+    cross-validation by Pareto-smoothed importance sampling (Vehtari, Gelman & Gabry 2017), with the Pareto shape k of
+    every frequency, as ArviZ's ``psislw`` with r_eff = 1.  theta (B, n, ndim) with n >= 2, w (N,) or (B, N), y, yerr
+    (B, 2, N) -> dict of ``elpd_i``, ``p_i``, ``pareto_k`` (B, N), ``elpd``, ``p_loo``, ``se`` (B,) float64 and
+    ``n_high_k`` (B,) int32.  ll[s, j] is ``waic``'s pointwise log-likelihood; elpd_i[j] = logsumexp_s(xt + ll) -
+    logsumexp_s(xt) with xt the smoothed log importance ratios, p_i = lppd - elpd_i, elpd = sum_j elpd_i,
+    p_loo = sum_j p_i, se = sqrt(N var_j(elpd_i, ddof=1)), n_high_k = #{j : k_j > min(1 - 1/log10 n, 0.7)} (k = inf when
+    the tail has 4 samples or fewer).  Z in FP64 for every ``precision``; a NaN sample makes its spectrum all-NaN.
+    Two launches per 65,535 spectra."""
+    lib = _lib.load()
+    _chk_cuda_f64(theta, w, y, yerr, spec.taus, spec.log_taus)
+    B, n, ndim = theta.shape
+    N = w.shape[-1]
+    if ndim != spec.ndim or tuple(y.shape) != (B, 2, N) or tuple(yerr.shape) != (B, 2, N):
+        raise ValueError(f"psis_loo: theta (B, n, {spec.ndim}) and y, yerr (B, 2, {N}) expected")
+    dev = theta.device
+    f64 = dict(dtype=torch.float64, device=dev)
+    out = dict(elpd_i=torch.empty((B, N), **f64), p_i=torch.empty((B, N), **f64), pareto_k=torch.empty((B, N), **f64),
+               elpd=torch.empty((B,), **f64), p_loo=torch.empty((B,), **f64), se=torch.empty((B,), **f64),
+               n_high_k=torch.empty((B,), dtype=torch.int32, device=dev))
+    d = spec.desc(N)
+    ts = spec.tau_stride()
+    for s0 in range(0, B, 65535):                  # one call per 65,535 spectra
+        k = min(65535, B - s0)
+        sl = slice(s0, s0 + k)
+        taus = spec.taus if ts == 0 else spec.taus[sl]
+        lts = spec.log_taus if ts == 0 else spec.log_taus[sl]
+        rc = lib.bisip_psis_loo(C.byref(d), k, n, _lib.ptr(theta[sl]), _lib.ptr(w if w.dim() == 1 else w[sl]),
+                                _w_stride(w), _lib.ptr(taus), _lib.ptr(lts), ts, _lib.ptr(y[sl]), _lib.ptr(yerr[sl]),
+                                *[_lib.ptr(out[key][sl]) for key in ('elpd_i', 'p_i', 'pareto_k', 'elpd', 'p_loo', 'se',
+                                                                       'n_high_k')],
+                                _lib.stream_ptr(dev))
+        _lib.check(rc, "bisip_psis_loo")
+    return out

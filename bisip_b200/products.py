@@ -54,7 +54,9 @@ def batch_table(param_names, results, ids=None, percentiles=(2.5, 50, 97.5)):
     ``autocorr_time`` (``fit(..., autocorr=True)``) — one ``<name>_tau`` column per parameter, then — when they hold the
     total chargeability (``fit(..., rtd=True)``) — ``total_m_mean``, ``total_m_std`` and one ``total_m_p<q>`` per
     percentile, then — when they hold the WAIC (``fit(..., waic=True)``) — ``elpd_waic``, ``p_waic``, ``se_elpd_waic``
-    and ``waic_n_high_p``.  The RTD, model-curve and pointwise WAIC arrays stay in ``results``."""
+    and ``waic_n_high_p``, then — when they hold PSIS-LOO (``fit(..., loo=True)``) — ``elpd_loo``, ``p_loo``,
+    ``se_elpd_loo`` and ``loo_n_high_k``.  The RTD, model-curve, pointwise WAIC / LOO and Pareto-k arrays stay in
+    ``results``."""
     B = results['mean'].shape[0]
     ids = np.arange(B) if ids is None else np.asarray(ids)
     cols = ['spectrum', 'acceptance_fraction', 'flags']
@@ -77,6 +79,10 @@ def batch_table(param_names, results, ids=None, percentiles=(2.5, 50, 97.5)):
         cols += ['elpd_waic', 'p_waic', 'se_elpd_waic', 'waic_n_high_p']
         blocks += [results['elpd_waic'][:, None], results['p_waic'][:, None], results['se_elpd_waic'][:, None],
                    results['waic_n_high_p'].astype(np.float64)[:, None]]
+    if 'elpd_loo' in results:
+        cols += ['elpd_loo', 'p_loo', 'se_elpd_loo', 'loo_n_high_k']
+        blocks += [results['elpd_loo'][:, None], results['p_loo'][:, None], results['se_elpd_loo'][:, None],
+                   results['loo_n_high_k'].astype(np.float64)[:, None]]
     return cols, np.concatenate(blocks, axis=1)
 
 
@@ -87,12 +93,27 @@ def compare_waic(res_a, res_b):
     Gelman & Gabry 2017), each of shape (B,) (scalars for single-spectrum dicts).  The comparison is only meaningful for
     two fits of the same ``zn`` / ``zn_err``: the pointwise terms are paired by frequency.  Raises ``ValueError`` when
     the shapes differ."""
-    ea, eb = np.asarray(res_a['elpd_waic'], dtype=np.float64), np.asarray(res_b['elpd_waic'], dtype=np.float64)
-    pa = np.asarray(res_a['waic_pointwise'], dtype=np.float64)
-    pb = np.asarray(res_b['waic_pointwise'], dtype=np.float64)
+    return _compare_elpd(res_a, res_b, 'compare_waic', 'elpd_waic', 'waic_pointwise')
+
+
+def compare_loo(res_a, res_b):
+    """Spectrum-by-spectrum PSIS-LOO comparison of two fits (``fit(..., loo=True)`` results, or ``get_loo`` dicts):
+    ``elpd_diff`` = elpd_loo_a - elpd_loo_b (positive: model a is expected to predict the data better) and ``se_diff``
+    = sqrt(N var_j(loo_pointwise_a - loo_pointwise_b, ddof=1)), the standard error of that difference (Vehtari, Gelman &
+    Gabry 2017), each of shape (B,) (scalars for single-spectrum dicts).  As ``compare_waic``: only meaningful for two
+    fits of the same ``zn`` / ``zn_err``; raises ``ValueError`` when the shapes differ.  Check ``pareto_k`` first: a
+    frequency with a high k makes its elpd_loo term unreliable."""
+    return _compare_elpd(res_a, res_b, 'compare_loo', 'elpd_loo', 'loo_pointwise')
+
+
+def _compare_elpd(res_a, res_b, name, total, pointwise):
+    """elpd difference and its standard error from the per-spectrum totals and the per-frequency pointwise terms."""
+    ea, eb = np.asarray(res_a[total], dtype=np.float64), np.asarray(res_b[total], dtype=np.float64)
+    pa = np.asarray(res_a[pointwise], dtype=np.float64)
+    pb = np.asarray(res_b[pointwise], dtype=np.float64)
     if ea.shape != eb.shape or pa.shape != pb.shape or pa.shape[:-1] != ea.shape:
-        raise ValueError(f"compare_waic: shapes differ (elpd_waic {ea.shape} vs {eb.shape}, "
-                         f"waic_pointwise {pa.shape} vs {pb.shape})")
+        raise ValueError(f"{name}: shapes differ ({total} {ea.shape} vs {eb.shape}, "
+                         f"{pointwise} {pa.shape} vs {pb.shape})")
     d = pa - pb
     N = d.shape[-1]
     return {'elpd_diff': ea - eb, 'se_diff': np.sqrt(N * np.var(d, axis=-1, ddof=1))}

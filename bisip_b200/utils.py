@@ -51,6 +51,24 @@ class utils(object):
         return {'elpd_waic': float(r['elpd']), 'p_waic': float(r['p_waic']), 'se_elpd_waic': float(r['se']),
                 'waic_pointwise': r['lppd'] - r['p'], 'waic_n_high_p': int(r['n_high_p'])}
 
+    def get_loo(self, chain=None, **kwargs):
+        """PSIS-LOO of the fit over an MCMC chain: leave-one-out cross-validation by Pareto-smoothed importance sampling
+        (Vehtari, Gelman & Gabry 2017; ArviZ's ``psislw`` with r_eff = 1), for comparing models fitted to the same data
+        where WAIC is unreliable.  A dict of ``elpd_loo``, ``p_loo``, ``se_elpd_loo`` (floats), ``loo_pointwise`` (N,)
+        = elpd_loo per frequency, ``pareto_k`` (N,), the Pareto shape of each frequency's importance ratios (inf for a
+        tail of 4 samples or fewer), and ``loo_n_high_k``, the number of frequencies with k > min(1 - 1/log10 S, 0.7).
+        The kernel behind ``BatchInversion.fit(..., loo=True)`` (``engine.psis_loo``), FP64 for every precision.
+        ``chain`` / ``discard`` / ``thin`` as in ``get_model_percentile``."""
+        chain = self.parse_chain(chain, **kwargs)
+        dev = _lib.require_cuda(getattr(self, "device", None))
+        th = _lib.dev_f64(chain, dev).reshape(1, -1, chain.shape[-1])
+        w = _lib.dev_const(self.data['w'], dev)
+        y = _lib.dev_f64(self.data['zn'], dev).reshape(1, 2, -1)
+        ye = _lib.dev_f64(self.data['zn_err'], dev).reshape(1, 2, -1)
+        r = {k: v[0].cpu().numpy() for k, v in engine.psis_loo(self._spec(dev), th, w, y, ye).items()}
+        return {'elpd_loo': float(r['elpd']), 'p_loo': float(r['p_loo']), 'se_elpd_loo': float(r['se']),
+                'loo_pointwise': r['elpd_i'], 'pareto_k': r['pareto_k'], 'loo_n_high_k': int(r['n_high_k'])}
+
     # ---------------------------------------------------------------- parameter statistics
     def _chain_stats(self, chain, p=None, mean=False, std=False):
         dev = _lib.require_cuda(getattr(self, "device", None))

@@ -26,6 +26,7 @@
  *   bisip_rtd_stats          <- relaxation_time_distribution / total_m of decomposition.ipynb
  *                               cells 25-29 over the chain, then np.percentile / mean / std
  *   bisip_waic               <- (no counterpart: the tutorials compare models by eye with plot_fit)
+ *   bisip_psis_loo           <- (no counterpart: the reference has no leave-one-out cross-validation)
  *
  * Layouts (all row-major, float64):
  *   theta   [n_spectra][n_theta][ndim]      parameter vectors (order as the reference's
@@ -259,6 +260,34 @@ int bisip_waic(const bisip_model_desc *desc, int n_spectra, int64_t n_theta, con
                const double *y, const double *yerr,
                double *lppd_out, double *p_out, double *elpd_out, double *p_waic_out, double *se_out,
                int32_t *n_high_p_out, void *stream);
+
+/*
+ * PSIS-LOO: leave-one-out cross-validation by Pareto-smoothed importance sampling (Vehtari, Gelman & Gabry 2017;
+ * Vehtari, Simpson, Gelman, Yao & Gabry 2024), with the Pareto shape k of every frequency, of every spectrum from its
+ * chain, read in place.  Arguments as bisip_waic; ll[s][j] is bisip_waic's pointwise log-likelihood and S = n_theta.
+ * For each frequency j, as ArviZ's psislw / _gpdfit / _gpinv with r_eff = 1:
+ *   x_s = -ll[s][j] - max_s(-ll[s][j]);  M = ceil(min(0.2 S, 3 sqrt(S)));  cutoff = max((M+1)-th largest x, ln DBL_MIN)
+ *   tail T = {s : x_s > cutoff}, L = |T|.  L <= 4: k = +inf, xt = x.  Otherwise (k, sigma) = the Zhang & Stephens
+ *   generalized Pareto fit of the ascending exp(x_T) - exp(cutoff) (with the weakly informative prior on k); if k is
+ *   finite the i-th smallest tail sample gets xt = ln(gpinv((i + 0.5) / L, k, sigma) + exp(cutoff)), then
+ *   xt = min(xt, 0); otherwise xt = x.
+ *   elpd_i_out[b][j] = logsumexp_s(xt + ll) - logsumexp_s(xt)     p_i_out[b][j] = lppd_j - elpd_i_out[b][j]
+ *   k_out[b][j]      = k                                          (lppd_j = logsumexp_s ll - ln S)
+ *   elpd_out[b]      = sum_j elpd_i                               p_loo_out[b] = sum_j p_i   (ascending j)
+ *   se_out[b]        = sqrt(N var_j(elpd_i, ddof=1))              n_high_k_out[b] = #{j : k_j > min(1 - 1/log10 S, 0.7)}
+ * Z is evaluated in FP64 for every desc->precision.  A NaN anywhere in a spectrum's samples makes all its outputs NaN
+ * (n_high_k 0).  Two launches: one CTA per (frequency, spectrum), then one thread per spectrum for the totals; fixed-order
+ * reductions: a spectrum's result depends on its own chain and data only.  No workspace.  A chain that fits one CTA's
+ * shared memory (S up to about 25,900 on a B200) is evaluated there once; a longer one is re-evaluated per pass, with
+ * only its Pareto tail (2M doubles) in shared memory.
+ * BISIP_ERR_BAD_ARG: as bisip_waic;
+ * BISIP_ERR_UNSUPPORTED: n_spectra > 65535, n_coef > 32, a tail that does not fit in shared memory (S above about 2e7).
+ */
+int bisip_psis_loo(const bisip_model_desc *desc, int n_spectra, int64_t n_theta, const double *theta,
+                   const double *w, int64_t w_stride, const double *taus, const double *log_taus, int64_t tau_stride,
+                   const double *y, const double *yerr,
+                   double *elpd_i_out, double *p_i_out, double *k_out, double *elpd_out, double *p_loo_out,
+                   double *se_out, int32_t *n_high_k_out, void *stream);
 
 #ifdef __cplusplus
 }
